@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the hot path: env-steps/s including the 64x64x3 render (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
     python bench.py --impl reference ...      # reference C++ engine (oracle/_ref) on the host cores
     python bench.py --game coinrun --envs-per-gpu 32768 [--max-episode-steps 32]   # one explicit workload
@@ -30,6 +30,11 @@ Per workload:
             plugin call itself, cenv_step of lib<Game>.so (ctypes, batched "action" in, "screen" out);
             `d2h_ceiling_gbs` = plain cudaMemcpyAsync of the observation bytes into pinned memory on this box, and
             `d2h_frac` = how much of that the pipelined path reaches;
+  --steps   K timed steps in every timed loop of every workload (device-resident, back to back, profiled, e2e, cenv);
+  --dump-outputs DIR   after the timed device-resident steps of each workload, what they handed the caller in the last
+            step, as float32 .npy files `<game>_<envs>[_ep<k>]_<array>.npy`: `obs` of a fixed, seeded sample of DUMP_ENVS
+            envs (`env_index` says which) and `reward` / `terminated` / `truncated` of every env (rank 0's shard). Inputs
+            (env seeds, action stream) are the same from run to run, so two builds can be compared array for array.
   roofline  dominant kernel (k_render) against the measured HBM copy bandwidth in MEASURED_PEAKS.json, algorithmic bytes
             = 12 297 B per env-step (SURVEY.md §8d); traffic = dram bytes of one launch from the committed ncu capture
             (profiles/traffic.json) when one exists for the workload.
@@ -54,6 +59,8 @@ UNIT = "env-steps/s"
 BASE_SEED = 0
 BURN_IN = 300
 GAMES = ("bossfight", "caveflyer", "chaser", "climber", "coinrun", "jumper", "maze")
+
+DUMP_ENVS = 64   # 64 x 12 288 B x 4 (float32) = 3.1 MB of observations per workload, 11 workloads at most
 
 HEADLINE = dict(tag="configs[2]", game="bossfight", envs=16384, max_ep=0)
 SINGLE_GPU_EXTRA = [dict(tag="configs[0]", game="maze", envs=256, max_ep=0), dict(tag="configs[1]", game="coinrun", envs=4096, max_ep=0)]
@@ -250,6 +257,13 @@ def measure(c, w, steps, warmup, full):
             c.flush.zero_()
     c.barrier()
     out["wall_s"] = time.perf_counter() - wall0
+    if c.dump:
+        idx = np.sort(np.random.RandomState(0).choice(N, min(N, DUMP_ENVS), replace=False))
+        out["outputs"] = {"env_index": idx.astype(np.float32),
+                          "obs": obs[torch.from_numpy(idx).to(dev)].cpu().numpy().astype(np.float32),
+                          "reward": rew.cpu().numpy().astype(np.float32),
+                          "terminated": term.cpu().numpy().astype(np.float32),
+                          "truncated": trunc.cpu().numpy().astype(np.float32)}
     out["launches"] = env.kernel_launches - launches0
     out["dev_ms"] = sum(s.elapsed_time(e) for s, e in zip(starts, ends))
     out["resets_per_step"] = float(done_count.item()) / steps
@@ -266,7 +280,7 @@ def measure(c, w, steps, warmup, full):
         # ---- profiled pass: per-kernel CUDA events (eager launches)
         env.profile(True)
         with torch.cuda.stream(stream):
-            for t in range(min(steps, 50)):
+            for t in range(steps):
                 env.step_torch(actions[t % pool])
                 c.flush.zero_()
         c.barrier()
@@ -281,7 +295,7 @@ def measure(c, w, steps, warmup, full):
             r = torch.empty(N, dtype=torch.float32).pin_memory()
             d = torch.empty(N, dtype=torch.uint8).pin_memory()
             bufs.append((o.numpy(), r.numpy(), d.numpy(), (o, r, d)))
-        e2e_steps = max(10, min(steps, 60))
+        e2e_steps = steps
         out["e2e_steps"] = e2e_steps
         for t in range(3):
             env.step(host_actions[t % pool])
@@ -439,6 +453,8 @@ def main():
     ap.add_argument("--ref-inner", type=int, default=50, help="env steps per env per timed sample of the reference arm")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra", action="store_true", help="headline workload only (skip the other BASELINE configs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the timed path returned in its last step of each workload as DIR/<name>.npy")
     a = ap.parse_args()
     a.warmup = max(a.warmup, 3) if a.impl == "b200" else a.warmup
 
@@ -466,6 +482,7 @@ def main():
             os.environ["NCCL_DEBUG"] = "WARN"     # keep stdout to the one JSON line (no "NCCL version" banner)
         dist.init_process_group("nccl", device_id=c.dev)
     c.flush = torch.empty(256 << 20, dtype=torch.uint8, device=c.dev)
+    c.dump = a.dump_outputs is not None and rank == 0
 
     def barrier():
         torch.cuda.synchronize(c.dev)
@@ -478,6 +495,7 @@ def main():
     sampler.start()
     m = measure(c, headline, a.steps, a.warmup, True)
     head = summarise(c, headline, m, a.steps, a.warmup, True)
+    dumps = [(headline, m.get("outputs"))]
     extra = []
     if not a.game and not a.no_extra:
         todo = [(w, True) for w in SINGLE_GPU_EXTRA]
@@ -485,11 +503,18 @@ def main():
             todo += [(dict(tag="configs[3] slice", game=g, envs=32768 // world, max_ep=0), False) for g in GAMES]
             todo += [(dict(tag="configs[4] slice", game="coinrun", envs=32768, max_ep=32), False)]
         for w, full in todo:
-            k = min(a.steps, 60)
-            extra.append(summarise(c, w, measure(c, w, k, a.warmup, full), k, a.warmup, full))
+            m = measure(c, w, a.steps, a.warmup, full)
+            extra.append(summarise(c, w, m, a.steps, a.warmup, full))
+            dumps.append((w, m.get("outputs")))
     sampler.stop_flag = True
     sampler.join(timeout=2)
 
+    if c.dump:
+        os.makedirs(a.dump_outputs, exist_ok=True)
+        for w, arrays in dumps:
+            name = "%s_%d%s" % (w["game"], w["envs"], "_ep%d" % w["max_ep"] if w["max_ep"] else "")
+            for k, v in arrays.items():
+                np.save(os.path.join(a.dump_outputs, "%s_%s.npy" % (name, k)), v)
     if rank == 0:
         line = {"metric": METRIC, "value": head["value"], "unit": UNIT, "n_gpus": world, "steps": a.steps, "warmup": a.warmup,
                 "ms_per_step": head["ms_per_step"], "higher_is_better": True, "scaling": "weak", "vs_baseline": None,

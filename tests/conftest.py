@@ -15,16 +15,16 @@ def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box: pytest -m gpu)")
 
 
-@pytest.fixture(scope="session")
-def oracle_available():
-    """oracle/_ref is (re)built here when the reference sources are present; on the GPU box the
-    prebuilt libraries travel with the working tree."""
-    from oracle import build_ref, ref_env
-    try:
-        build_ref.build()
-    except Exception:
-        pass
-    return ref_env.available()
+@pytest.fixture
+def reference(request):
+    """Reference environments for a parity test (tests/reference.py): the compiled reference when oracle/_ref is built,
+    else the host-sim stand-in; what they return is checked against the test's recorded tape when it ends."""
+    from oracle import build_ref
+    from tests.reference import Reference
+    build_ref.build()
+    ref = Reference(request.node.nodeid)
+    yield ref
+    ref.finish()
 
 
 def golden(game):

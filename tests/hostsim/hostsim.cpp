@@ -11,6 +11,7 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <map>
 #include <memory>
 #include <string>
 #include <vector>
@@ -40,8 +41,8 @@ struct Sim : SimBase {
     std::vector<char> state_mem, common_mem, arena;
     std::vector<uint8_t> view_cache;
     std::vector<uint32_t> mt_scratch;
-    std::vector<TexInfo> tex;
-    std::vector<uint32_t> atlas;
+    const TexInfo* tex = nullptr;
+    const uint32_t* atlas = nullptr;
     std::unique_ptr<FrameOf<G>> frame;
 
     bool init(int n, uint32_t base_seed, int max_ep, const char* assets, std::string* err, int mode = -1) {
@@ -58,13 +59,24 @@ struct Sim : SimBase {
         obs.assign((size_t)N * OBS_BYTES, 0); terminated.assign(N, 0); truncated.assign(N, 0); reward.assign(N, 0.0f);
         int ntex = 0;
         const char* const* names = G::texture_names(&ntex);
-        if (!load_textures(assets, names, ntex, &tex, &atlas, err)) return false;
-        frame_init_tiletex<G>(*frame, tex.data());
+        // decoding the textures dominates creation, and the parity tests create thousands of one-env sims
+        static std::map<std::pair<std::string, const char* const*>, std::pair<std::vector<TexInfo>, std::vector<uint32_t>>> loaded;
+        auto key = std::make_pair(std::string(assets ? assets : ""), names);
+        auto it = loaded.find(key);
+        if (it == loaded.end()) {
+            std::vector<TexInfo> t;
+            std::vector<uint32_t> a;
+            if (!load_textures(assets, names, ntex, &t, &a, err)) return false;
+            it = loaded.emplace(key, std::make_pair(std::move(t), std::move(a))).first;
+        }
+        tex = it->second.first.data();
+        atlas = it->second.second.data();
+        frame_init_tiletex<G>(*frame, tex);
         for (int e = 0; e < N; e++) seed_body(c, e, base_seed + (uint32_t)e, true);
         for (int e = 0; e < N; e++) reset_body<G>(st, c, e, mt_scratch.data(), arena.data(), 0);
         return true;
     }
-    void render(int e) { render_body<G>(st, c, e, *frame, tex.data(), atlas.data(), obs.data(), G::STATIC_VIEW ? view_cache.data() : nullptr); }
+    void render(int e) { render_body<G>(st, c, e, *frame, tex, atlas, obs.data(), G::STATIC_VIEW ? view_cache.data() : nullptr); }
     void reset_all(const int32_t* seeds) override {
         for (int e = 0; e < N; e++) {
             if (seeds) seed_body(c, e, (uint32_t)seeds[e], false);
@@ -84,7 +96,7 @@ struct Sim : SimBase {
         return st.find(name, ptr, esz, pe) || c.find(name, ptr, esz, pe);
     }
     void render_human(int env, int width, int height, uint8_t* out) override {
-        render_human_body<G>(st, c, env, *frame, tex.data(), atlas.data(), out, width, height, 0, width * height);
+        render_human_body<G>(st, c, env, *frame, tex, atlas, out, width, height, 0, width * height);
     }
 };
 

@@ -19,7 +19,7 @@ class _Raw:
         self.__cuda_array_interface__ = {"shape": shape, "typestr": typestr, "data": (ptr, False), "version": 2}
 
 
-def test_cenv_device_pointers_and_host_copy_off(oracle_available):
+def test_cenv_device_pointers_and_host_copy_off(reference):
     """A cenv.py-style caller gets the observations WITHOUT the device -> host copy: make-option host_copy = 0, the device
     addresses arrive as INT-pair infos of reset / step and through the exported cenv_device_buffer; the data behind them
     equals the host-copy path and the live oracle."""
@@ -48,11 +48,8 @@ def test_cenv_device_pointers_and_host_copy_off(oracle_available):
     reward = torch.as_tensor(_Raw(_ptr(ib, "reward_device"), (n,), "<f4"), device=dev)
     np.testing.assert_array_equal(screen.cpu().numpy().reshape(-1), oa["screen"])
     assert not ob["screen"].any()      # host_copy = 0: the host "screen" buffer is never written
-    refs = None
-    if oracle_available:
-        from oracle import ref_env
-        refs = [ref_env.RefEnv("coinrun", seed + i) for i in range(n)]
-        np.testing.assert_array_equal(screen.cpu().numpy(), np.stack([r.reset() for r in refs]))
+    refs = [reference.RefEnv("coinrun", seed + i) for i in range(n)]
+    np.testing.assert_array_equal(screen.cpu().numpy(), np.stack([r.reset() for r in refs]))
     for t in range(T):
         oa, _, _, _, ia = a.step(acts[t])
         ob, _, _, _, ib = b.step(acts[t])
@@ -61,12 +58,11 @@ def test_cenv_device_pointers_and_host_copy_off(oracle_available):
         np.testing.assert_array_equal(reward.cpu().numpy(), ia["reward"])
         np.testing.assert_array_equal(ib["reward"], ia["reward"])            # rewards / flags are still copied
         np.testing.assert_array_equal(ib["terminated"], ia["terminated"])
-        if refs:
-            ro = []
-            for i, r in enumerate(refs):
-                o, w, d = r.step(acts[t, i])
-                ro.append(r.reset() if d else o)
-            np.testing.assert_array_equal(screen.cpu().numpy(), np.stack(ro), err_msg="oracle, step %d" % t)
+        ro = []
+        for i, r in enumerate(refs):
+            o, w, d = r.step(acts[t, i])
+            ro.append(r.reset() if d else o)
+        np.testing.assert_array_equal(screen.cpu().numpy(), np.stack(ro), err_msg="oracle, step %d" % t)
     a.close(); b.close()
 
 
@@ -83,7 +79,7 @@ def test_cenv_single_env_reports_no_infos():
 
 
 @pytest.mark.parametrize("game,mode", [("coinrun", None), ("chaser", None), ("chaser", "extreme"), ("maze", "easy")])
-def test_vector_env_matches_oracle(game, mode, oracle_available):
+def test_vector_env_matches_oracle(game, mode, reference):
     """ProcgenVectorEnv: zero-copy tensors, actions as CUDA tensor / numpy / list, same-step autoreset, seeds, and the
     `distribution_mode` keyword by name."""
     import torch
@@ -99,30 +95,26 @@ def test_vector_env_matches_oracle(game, mode, oracle_available):
     obs, info = env.reset()
     assert obs.is_cuda and obs.dtype == torch.uint8 and tuple(obs.shape) == (n, 64, 64, 3) and info == {}
     assert obs.data_ptr() == env.env.torch_views()[0].data_ptr()     # a view of the engine's buffer, not a copy
-    refs = None
-    if oracle_available:
-        from oracle import ref_env
-        refs = [ref_env.RefEnv(game, seed + i, mode=ProcgenVectorEnv.DISTRIBUTION_MODES[mode] if mode else None) for i in range(n)]
-        np.testing.assert_array_equal(obs.cpu().numpy(), np.stack([r.reset() for r in refs]))
+    refs = [reference.RefEnv(game, seed + i, mode=ProcgenVectorEnv.DISTRIBUTION_MODES[mode] if mode else None) for i in range(n)]
+    np.testing.assert_array_equal(obs.cpu().numpy(), np.stack([r.reset() for r in refs]))
     age = np.zeros(n, np.int64)
     for t in range(T):
         a = acts[t]
         arg = torch.from_numpy(a).cuda() if t % 3 == 0 else (a if t % 3 == 1 else a.tolist())
         obs, rew, term, trunc, info = env.step(arg)
         assert rew.dtype == torch.float32 and term.dtype == torch.bool and trunc.dtype == torch.bool
-        if refs:
-            ro, rr, rd, rt = [], [], [], []
-            for i, r in enumerate(refs):
-                o, w, d = r.step(a[i])
-                age[i] += 1
-                tr = (not d) and age[i] >= 25
-                if d or tr:
-                    o = r.reset(); age[i] = 0
-                ro.append(o); rr.append(w); rd.append(d); rt.append(tr)
-            np.testing.assert_array_equal(obs.cpu().numpy(), np.stack(ro), err_msg="pixels, step %d" % t)
-            np.testing.assert_array_equal(rew.cpu().numpy(), np.array(rr, np.float32))
-            np.testing.assert_array_equal(term.cpu().numpy(), np.array(rd))
-            np.testing.assert_array_equal(trunc.cpu().numpy(), np.array(rt))
+        ro, rr, rd, rt = [], [], [], []
+        for i, r in enumerate(refs):
+            o, w, d = r.step(a[i])
+            age[i] += 1
+            tr = (not d) and age[i] >= 25
+            if d or tr:
+                o = r.reset(); age[i] = 0
+            ro.append(o); rr.append(w); rd.append(d); rt.append(tr)
+        np.testing.assert_array_equal(obs.cpu().numpy(), np.stack(ro), err_msg="pixels, step %d" % t)
+        np.testing.assert_array_equal(rew.cpu().numpy(), np.array(rr, np.float32))
+        np.testing.assert_array_equal(term.cpu().numpy(), np.array(rd))
+        np.testing.assert_array_equal(trunc.cpu().numpy(), np.array(rt))
     # interchange: DLPack capsules and __cuda_array_interface__ alias the same memory
     caps = env.dlpack()
     assert torch.utils.dlpack.from_dlpack(caps[0]).data_ptr() == obs.data_ptr()
@@ -137,18 +129,15 @@ def test_vector_env_matches_oracle(game, mode, oracle_available):
 
 @pytest.mark.parametrize("game,mode", [("coinrun", None), ("bossfight", None), ("jumper", None), ("maze", None),
                                        ("chaser", 2), ("caveflyer", 2)])
-def test_cenv_render_matches_oracle(game, mode, oracle_available):
+def test_cenv_render_matches_oracle(game, mode, reference):
     """cenv_render of the drop-in library = the reference's human-mode frame (512x512 default window and a custom size),
     rendered on the device; with the make-option "distribution_mode" passed through the cenv options for two of the
     instantiations that have their own world size."""
-    if not oracle_available:
-        pytest.skip("oracle/_ref did not travel")
-    from oracle import ref_env
     from procgen2_b200.build import game_lib_path
     from procgen2_b200.cenv import CEnv
     for opts in ({}, {"width": 200, "height": 200}):
         env = CEnv(game_lib_path(game), options=dict(seed=515, **opts, **({} if mode is None else {"distribution_mode": mode})))
-        ref = ref_env.RefEnv(game, 515, mode=mode, **opts)
+        ref = reference.RefEnv(game, 515, mode=mode, **opts)
         obs, _ = env.reset()
         np.testing.assert_array_equal(obs["screen"].reshape(64, 64, 3), ref.reset())
         rs = np.random.RandomState(1)
@@ -167,21 +156,18 @@ def test_cenv_render_matches_oracle(game, mode, oracle_available):
 
 
 @pytest.mark.parametrize("game", ["climber", "bossfight"])
-def test_distribution_mode_option(game, oracle_available):
+def test_distribution_mode_option(game, reference):
     """cenv make-option "distribution_mode" = 0 (easy) on the GPU against the reference with its compile-time mode flipped
     through the probe (climber: Config::easy_mode; bossfight: System_Mob_AI::Config::mode); a (game, mode) pair that is
     not built is refused loudly."""
     from procgen2_b200.engine import BatchedEnv
     with pytest.raises(RuntimeError, match="distribution_mode"):
         BatchedEnv("climber", 4, distribution_mode=2)     # climber has no third mode
-    if not oracle_available:
-        pytest.skip("oracle/_ref did not travel")
-    from oracle import ref_env
     n, seed, T, ep = (32, 9100, 90, 30) if game == "climber" else (12, 9100, 500, 250)
     rs = np.random.RandomState(12)
     acts = rs.randint(0, 15, size=(T, n)).astype(np.int32)
     env = BatchedEnv(game, n, seed=seed, max_episode_steps=ep, distribution_mode=0)
-    refs = [ref_env.RefEnv(game, seed + i, **(dict(easy_mode=True) if game == "climber" else dict(mode=0))) for i in range(n)]
+    refs = [reference.RefEnv(game, seed + i, **(dict(easy_mode=True) if game == "climber" else dict(mode=0))) for i in range(n)]
     env.reset()
     np.testing.assert_array_equal(env.fetch()[0], np.stack([r.reset() for r in refs]))
     age = np.zeros(n, np.int64)
@@ -204,19 +190,16 @@ def test_distribution_mode_option(game, oracle_available):
                                                     ("chaser", 1, 13, 120, 300), ("chaser", 2, 19, 120, 300),
                                                     ("jumper", 0, 20, 100, 250), ("caveflyer", 0, 20, 100, 250),
                                                     ("jumper", 2, 45, 100, 250), ("caveflyer", 2, 45, 100, 250)])
-def test_world_size_modes(game, mode, dim, max_ep, T, oracle_available):
+def test_world_size_modes(game, mode, dim, max_ep, T, reference):
     """Distribution modes with their own world size = own instantiations (maze easy 15x15 / memory 31x31 with an agent-centred
     8x8 view: MazeT<MODE>; chaser hard 13x13 / extreme 19x19 with 5 enemies and 5 orbs: ChaserT<MODE>; jumper / caveflyer easy 20x20 and memory 45x45 with the unpruned cave), against the reference
     with its compile-time Config::mode set: tile maps + RNG after make, pixels / rewards / dones over truncated episodes."""
-    if not oracle_available:
-        pytest.skip("oracle/_ref did not travel")
-    from oracle import ref_env
     from procgen2_b200.engine import BatchedEnv
     n, seed = 48, 8300 + mode
     rs = np.random.RandomState(mode)
     acts = rs.randint(0, 15, size=(T, n)).astype(np.int32)
     env = BatchedEnv(game, n, seed=seed, max_episode_steps=max_ep, distribution_mode=mode)
-    refs = [ref_env.RefEnv(game, seed + i, mode=mode) for i in range(n)]
+    refs = [reference.RefEnv(game, seed + i, mode=mode) for i in range(n)]
     tb, _, pe = env.read_field("tiles")
     tiles = tb.reshape(n, pe)
     for i, r in enumerate(refs):

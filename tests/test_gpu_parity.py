@@ -1,7 +1,7 @@
 """GPU tests (pytest -m gpu on a B200): the CUDA engine, driven through its C ABI
 (libprocgen2_b200.so via ctypes) and through the per-game cenv drop-in libraries, against
-(1) the committed golden vectors generated from the compiled reference, (2) the live reference
-(oracle/_ref, when it travelled to the box), (3) size-independent properties at BASELINE sizes.
+(1) the committed golden vectors generated from the compiled reference, (2) reference environments
+(tests/reference.py: live when oracle/_ref is built, else the stand-in checked against recorded tapes), (3) size-independent properties at BASELINE sizes.
 Everything is bit-exact: rewards, terminated, pixels, tile maps, MT19937 state."""
 import numpy as np
 import pytest
@@ -46,14 +46,11 @@ def test_golden(game, stream):
 
 
 @pytest.mark.parametrize("game", IMPLEMENTED)
-def test_live_oracle(game, oracle_available):
-    if not oracle_available:
-        pytest.skip("oracle/_ref did not travel")
-    from oracle import ref_env
+def test_live_oracle(game, reference):
     n, T, seed = 48, 400, 900
     rs = np.random.RandomState(11)
     acts = np.where(rs.rand(T, n) < 0.5, rs.randint(0, 15, size=(T, n)), rs.choice([6, 7, 8, 8, 5], size=(T, n))).astype(np.int32)
-    refs = [ref_env.RefEnv(game, seed + i) for i in range(n)]
+    refs = [reference.RefEnv(game, seed + i) for i in range(n)]
     a = EngineAdapter(game, n, seed)
     episodes = check_against_oracle(a, refs, acts, tag=game)
     assert episodes > 0     # the auto-reset path was exercised

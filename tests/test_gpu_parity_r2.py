@@ -20,13 +20,6 @@ pytestmark = pytest.mark.gpu
 THREAD_PER_ENV_GAMES = ["maze", "bossfight", "caveflyer", "jumper"]   # G::LANE_AWARE == false: step_epw > 1 exists
 
 
-def _need_oracle(oracle_available):
-    if not oracle_available:
-        pytest.skip("oracle/_ref did not travel")
-    from oracle import ref_env
-    return ref_env
-
-
 def _mixed_actions(rs, T, n):
     return np.where(rs.rand(T, n) < 0.5, rs.randint(0, 15, size=(T, n)), rs.choice([6, 7, 8, 8, 5], size=(T, n))).astype(np.int32)
 
@@ -61,8 +54,7 @@ def _check_state(env, refs, idx=None, tag=""):
 
 @pytest.mark.parametrize("epw", [2, 4, 32])
 @pytest.mark.parametrize("game", THREAD_PER_ENV_GAMES)
-def test_step_epw_live_oracle(game, epw, oracle_available, monkeypatch):
-    ref_env = _need_oracle(oracle_available)
+def test_step_epw_live_oracle(game, epw, reference, monkeypatch):
     from procgen2_b200.engine import BatchedEnv
     from tests.parity_util import check_against_oracle
     from tests.test_gpu_parity import EngineAdapter
@@ -72,7 +64,7 @@ def test_step_epw_live_oracle(game, epw, oracle_available, monkeypatch):
     a = EngineAdapter(game, n, seed)
     monkeypatch.delenv("PG2_STEP_EPW")
     assert a.env.step_epw == epw
-    refs = [ref_env.RefEnv(game, seed + i) for i in range(n)]
+    refs = [reference.RefEnv(game, seed + i) for i in range(n)]
     episodes = check_against_oracle(a, refs, acts, tag="%s epw=%d" % (game, epw))
     _check_state(a.env, refs, tag=game)
     _assert_no_fault(a.env)
@@ -82,10 +74,9 @@ def test_step_epw_live_oracle(game, epw, oracle_available, monkeypatch):
     a.env.close()
 
 
-def test_bossfight_16384_sampled_oracle(oracle_available):
+def test_bossfight_16384_sampled_oracle(reference):
     """BASELINE configs[2] as the engine runs it (16 384 envs, warp-per-env step with the bullet rings on the lanes):
     64 sampled envs, 50 steps, against reference processes with the same seeds."""
-    ref_env = _need_oracle(oracle_available)
     from procgen2_b200.engine import BatchedEnv
     n, T, seed = 16384, 50, 7
     rs = np.random.RandomState(8)
@@ -95,7 +86,7 @@ def test_bossfight_16384_sampled_oracle(oracle_available):
     idx = np.sort(rs.choice(n, 64, replace=False))
     idx[:4] = [0, 1, n - 2, n - 1]
     idx = np.unique(idx)
-    refs = [ref_env.RefEnv("bossfight", seed + int(i)) for i in idx]
+    refs = [reference.RefEnv("bossfight", seed + int(i)) for i in idx]
     env.reset()
     np.testing.assert_array_equal(env.fetch()[0][idx], np.stack([r.reset() for r in refs]))
     for t in range(T):
@@ -121,14 +112,13 @@ def test_bossfight_16384_sampled_oracle(oracle_available):
 
 @pytest.mark.parametrize("max_ep", [1, 3, 8, 32])
 @pytest.mark.parametrize("game", IMPLEMENTED)
-def test_truncation_live_oracle(game, max_ep, oracle_available):
-    ref_env = _need_oracle(oracle_available)
+def test_truncation_live_oracle(game, max_ep, reference):
     from procgen2_b200.engine import BatchedEnv
     n, seed = 32, 2100 + max_ep
     T = max(24, 21 * max_ep)     # >= 21 episodes per env
     acts = _mixed_actions(np.random.RandomState(60 + max_ep), T, n)
     env = BatchedEnv(game, n, seed=seed, max_episode_steps=max_ep)
-    refs = [ref_env.RefEnv(game, seed + i) for i in range(n)]
+    refs = [reference.RefEnv(game, seed + i) for i in range(n)]
     env.reset()
     np.testing.assert_array_equal(env.fetch()[0], np.stack([r.reset() for r in refs]), err_msg="reset frame")
     age = np.zeros(n, np.int64)
@@ -161,8 +151,7 @@ def test_truncation_live_oracle(game, max_ep, oracle_available):
 
 # ---- (c) maze timeout -----------------------------------------------------------------------------------------------------
 
-def test_maze_timeout_live_oracle(oracle_available):
-    ref_env = _need_oracle(oracle_available)
+def test_maze_timeout_live_oracle(reference):
     from tests.parity_util import check_against_oracle
     from tests.test_gpu_parity import EngineAdapter
     n, T, seed = 48, 520, 3100
@@ -170,7 +159,7 @@ def test_maze_timeout_live_oracle(oracle_available):
     acts = rs.randint(0, 15, size=(T, n)).astype(np.int32)
     acts[:, : n // 2] = 4          # half of the envs never move: their episodes can only end by the 500-step timeout
     a = EngineAdapter("maze", n, seed)
-    refs = [ref_env.RefEnv("maze", seed + i) for i in range(n)]
+    refs = [reference.RefEnv("maze", seed + i) for i in range(n)]
     episodes = check_against_oracle(a, refs, acts, tag="maze timeout")
     assert episodes >= n // 2
     _check_state(a.env, refs, tag="maze timeout")
@@ -186,11 +175,10 @@ OTHER_MODES = [("maze", 0), ("maze", 2), ("chaser", 1), ("chaser", 2), ("jumper"
 
 
 @pytest.mark.parametrize("game,mode", [(g, None) for g in IMPLEMENTED] + OTHER_MODES)
-def test_gpu_level_generation_many_seeds(game, mode, oracle_available):
+def test_gpu_level_generation_many_seeds(game, mode, reference):
     """The warp-parallel generators (ordered BFS with atomicMin claims, unordered_set regrouping, bit-row automaton) exist
     only in the GPU build: 512 seeds x (make + 4 resets), tile map + complete RNG state + the reset frame every time
     (128 seeds for the distribution modes that have their own world size)."""
-    ref_env = _need_oracle(oracle_available)
     from procgen2_b200.engine import BatchedEnv
     n, seed, chunk = (512 if mode is None else 128), 52000, 128
     env = BatchedEnv(game, n, seed=seed, distribution_mode=-1 if mode is None else mode)
@@ -211,7 +199,7 @@ def test_gpu_level_generation_many_seeds(game, mode, oracle_available):
     _assert_no_fault(env)
     env.close()
     for c0 in range(0, n, chunk):
-        refs = [ref_env.RefEnv(game, seed + i, mode=mode) for i in range(c0, min(n, c0 + chunk))]
+        refs = [reference.RefEnv(game, seed + i, mode=mode) for i in range(c0, min(n, c0 + chunk))]
         for rnd in range(5):
             mt, mti, tiles = fields[rnd]
             for k, r in enumerate(refs):
@@ -290,17 +278,16 @@ def test_prefetch_when_every_env_finishes_every_step(game, n, max_ep, monkeypatc
 # ---- bossfight past its first seconds -----------------------------------------------------------------------------------
 
 @pytest.mark.parametrize("mode", [None, 0])
-def test_bossfight_whole_fight_live_oracle(mode, oracle_available):
+def test_bossfight_whole_fight_live_oracle(mode, reference):
     """The lane-aware k_step<bossfight> (bullet rings as visited prefixes, ballots over 8-lane groups) through whole fights:
     a policy that dodges and fires (random actions die within ~50 steps) walks the boss through its shielded / unshielded
     phases, every attack pattern, the shield bounces, hp and its death — pixels, rewards, dones every step, RNG at the end."""
-    ref_env = _need_oracle(oracle_available)
     from procgen2_b200.engine import BatchedEnv
     from tests.test_hostsim_parity import bossfight_policy
     n, seed, T = 16, 777, 1500
     rs = np.random.RandomState(seed)
     env = BatchedEnv("bossfight", n, seed=seed, distribution_mode=-1 if mode is None else mode)
-    refs = [ref_env.RefEnv("bossfight", seed + i, mode=mode) for i in range(n)]
+    refs = [reference.RefEnv("bossfight", seed + i, mode=mode) for i in range(n)]
     env.reset()
     np.testing.assert_array_equal(env.fetch()[0], np.stack([r.reset() for r in refs]))
     wins, longest, age = 0, 0, np.zeros(n, np.int64)
@@ -328,16 +315,15 @@ def test_bossfight_whole_fight_live_oracle(mode, oracle_available):
 # ---- chaser with orbs and eaten mobs --------------------------------------------------------------------------------------
 
 @pytest.mark.parametrize("mode", [None, 2])
-def test_chaser_orbs_and_eaten_mobs_live_oracle(mode, oracle_available):
+def test_chaser_orbs_and_eaten_mobs_live_oracle(mode, reference):
     """The warp-per-env k_step<chaser> (point loop on the lanes, votes for "ate an orb") with a corridor-walking policy: the
     agent covers the maze, eats orbs (mobs flee and slow down) and now and then a mob (respawn on a free cell drawn from the
     RNG, SURVEY Q17) — paths uniform-random actions hardly reach. Easy 11x11 and extreme 19x19."""
-    ref_env = _need_oracle(oracle_available)
     from procgen2_b200.engine import BatchedEnv
     n, seed, T = 16, 555, 1500
     rs = np.random.RandomState(seed)
     env = BatchedEnv("chaser", n, seed=seed, distribution_mode=-1 if mode is None else mode)
-    refs = [ref_env.RefEnv("chaser", seed + i, mode=mode) for i in range(n)]
+    refs = [reference.RefEnv("chaser", seed + i, mode=mode) for i in range(n)]
     env.reset()
     np.testing.assert_array_equal(env.fetch()[0], np.stack([r.reset() for r in refs]))
     cur = rs.choice([1, 7, 3, 5], size=n)
@@ -367,11 +353,10 @@ def test_chaser_orbs_and_eaten_mobs_live_oracle(mode, oracle_available):
 # ---- purposeful action streams for the warp-per-env platformers ------------------------------------------------------------
 
 @pytest.mark.parametrize("game,bias", [("coinrun", [8, 8, 7, 7, 5, 8, 6, 1, 4, 8]), ("climber", [2, 5, 8, 8, 2, 5, 1, 7, 5, 5])])
-def test_biased_actions_live_oracle(game, bias, oracle_available):
+def test_biased_actions_live_oracle(game, bias, reference):
     """Run-right-and-jump (coinrun) / jump-a-lot (climber) action streams, held for 6 steps with 15 % noise: the agents get
     deep into their levels (crates, saws, lava, enemies, coins; 50x more rewarded steps than uniform-random actions), through
     the warp-per-env k_step with the entity loops on the lanes."""
-    ref_env = _need_oracle(oracle_available)
     from procgen2_b200.engine import BatchedEnv
     n, seed, T = 32, 31415, 800
     rs = np.random.RandomState(seed)
@@ -379,7 +364,7 @@ def test_biased_actions_live_oracle(game, bias, oracle_available):
     acts = np.repeat(run, 6, axis=0)[:T]
     acts = np.where(rs.rand(T, n) < 0.15, rs.randint(0, 15, size=(T, n)), acts).astype(np.int32)
     env = BatchedEnv(game, n, seed=seed)
-    refs = [ref_env.RefEnv(game, seed + i) for i in range(n)]
+    refs = [reference.RefEnv(game, seed + i) for i in range(n)]
     env.reset()
     np.testing.assert_array_equal(env.fetch()[0], np.stack([r.reset() for r in refs]))
     rewarded = 0
@@ -401,15 +386,14 @@ def test_biased_actions_live_oracle(game, bias, oracle_available):
     env.close()
 
 
-def test_bossfight_partial_last_warp_live_oracle(oracle_available):
+def test_bossfight_partial_last_warp_live_oracle(reference):
     """13 envs with 8 lanes each: the last warp of k_step<bossfight> holds ONE env and three idle lane groups."""
-    ref_env = _need_oracle(oracle_available)
     from tests.parity_util import check_against_oracle
     from tests.test_gpu_parity import EngineAdapter
     n, T, seed = 13, 200, 8100
     acts = _mixed_actions(np.random.RandomState(3), T, n)
     a = EngineAdapter("bossfight", n, seed)
-    refs = [ref_env.RefEnv("bossfight", seed + i) for i in range(n)]
+    refs = [reference.RefEnv("bossfight", seed + i) for i in range(n)]
     check_against_oracle(a, refs, acts, tag="bossfight 13 envs")
     _check_state(a.env, refs, tag="bossfight 13 envs")
     _assert_no_fault(a.env)

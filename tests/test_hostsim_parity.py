@@ -1,6 +1,6 @@
 """CPU tests: the engine's device SOURCE (compiled for the host by tests/hostsim, single lane)
-against the golden vectors generated from the compiled reference, and against the live
-reference when oracle/_ref is available. The product path (CUDA) is covered by test_gpu_parity."""
+against the golden vectors generated from the compiled reference, and against reference environments
+(tests/reference.py: live when oracle/_ref is built, else the stand-in checked against recorded tapes). The product path (CUDA) is covered by test_gpu_parity."""
 import numpy as np
 import pytest
 
@@ -38,14 +38,11 @@ def test_golden(game, stream):
 
 
 @pytest.mark.parametrize("game", IMPLEMENTED)
-def test_live_oracle(game, oracle_available):
-    if not oracle_available:
-        pytest.skip("oracle/_ref not built")
-    from oracle import ref_env
+def test_live_oracle(game, reference):
     n, T, seed = 8, 300, 77
     rs = np.random.RandomState(5)
     acts = np.where(rs.rand(T, n) < 0.5, rs.randint(0, 15, size=(T, n)), rs.choice([6, 7, 8, 8, 5], size=(T, n))).astype(np.int32)
-    refs = [ref_env.RefEnv(game, seed + i) for i in range(n)]
+    refs = [reference.RefEnv(game, seed + i) for i in range(n)]
     check_against_oracle(SimAdapter(game, n, seed), refs, acts, tag=game)
 
 
@@ -53,15 +50,12 @@ OTHER_MODES = [("maze", 0), ("maze", 2), ("chaser", 1), ("chaser", 2), ("jumper"
 
 
 @pytest.mark.parametrize("game,mode", [(g, None) for g in IMPLEMENTED] + OTHER_MODES)
-def test_level_generation_many_seeds(game, mode, oracle_available):
+def test_level_generation_many_seeds(game, mode, reference):
     """Level layouts + the complete MT19937 state for many seeds and consecutive resets — the compiled-in mode of every game
     and every distribution mode that has its own world size."""
-    if not oracle_available:
-        pytest.skip("oracle/_ref not built")
-    from oracle import ref_env
     n, seed = 24, 31337
     sim = SimAdapter(game, n, seed, distribution_mode=-1 if mode is None else mode)
-    refs = [ref_env.RefEnv(game, seed + i, mode=mode) for i in range(n)]
+    refs = [reference.RefEnv(game, seed + i, mode=mode) for i in range(n)]
     for rnd in range(4):
         f = sim.fields()
         for i, r in enumerate(refs):
@@ -88,18 +82,15 @@ def test_max_episode_steps_truncates():
 
 @pytest.mark.parametrize("game", IMPLEMENTED)
 @pytest.mark.parametrize("max_ep", [1, 5])
-def test_truncation_live_oracle(game, max_ep, oracle_available):
+def test_truncation_live_oracle(game, max_ep, reference):
     """max_episode_steps (BASELINE configs[4]) against the reference driven as "step; every k steps: reset()":
     pixels, rewards, terminated, truncated, and the RNG state + tile map at the end. (GPU twin with more envs,
     longer horizons and k up to 32: tests/test_gpu_parity_r2.py.)"""
-    if not oracle_available:
-        pytest.skip("oracle/_ref not built")
-    from oracle import ref_env
     n, seed, T = 3, 600 + max_ep, 8 * max_ep + 3
     rs = np.random.RandomState(9)
     acts = rs.randint(0, 15, size=(T, n)).astype(np.int32)
     sim = SimAdapter(game, n, seed, max_episode_steps=max_ep)
-    refs = [ref_env.RefEnv(game, seed + i) for i in range(n)]
+    refs = [reference.RefEnv(game, seed + i) for i in range(n)]
     np.testing.assert_array_equal(sim.reset(), np.stack([r.reset() for r in refs]))
     age = np.zeros(n, np.int64)
     for t in range(T):
@@ -122,15 +113,12 @@ def test_truncation_live_oracle(game, max_ep, oracle_available):
         r.close()
 
 
-def test_maze_timeout_live_oracle(oracle_available):
+def test_maze_timeout_live_oracle(reference):
     """maze.cpp:308-310: an env that never reaches the goal terminates at step 500."""
-    if not oracle_available:
-        pytest.skip("oracle/_ref not built")
-    from oracle import ref_env
     n, seed, T = 2, 41, 503
     acts = np.full((T, n), 4, np.int32)
     acts[:, 1] = np.random.RandomState(1).randint(0, 15, size=T)
-    refs = [ref_env.RefEnv("maze", seed + i) for i in range(n)]
+    refs = [reference.RefEnv("maze", seed + i) for i in range(n)]
     episodes = check_against_oracle(SimAdapter("maze", n, seed), refs, acts, tag="maze timeout")
     assert episodes >= 1
     for r in refs:
@@ -138,17 +126,14 @@ def test_maze_timeout_live_oracle(oracle_available):
 
 
 @pytest.mark.parametrize("game", IMPLEMENTED)
-def test_human_render_live_oracle(game, oracle_available):
+def test_human_render_live_oracle(game, reference):
     """cenv_render (render_game(false), coinrun.cpp:393-411): the scene drawn again with the window size as camera_size —
     square windows interleaved with stepping (the observations must not be disturbed), a non-square one at the end
     (there the reference's own step logic would afterwards see the window aspect, SURVEY Q11: not interleaved)."""
-    if not oracle_available:
-        pytest.skip("oracle/_ref not built")
-    from oracle import ref_env
     n, seed = 2, 77
     for (W, H) in ((96, 96), (160, 100)):
         sim = SimAdapter(game, n, seed)
-        refs = [ref_env.RefEnv(game, seed + i, width=W, height=H) for i in range(n)]
+        refs = [reference.RefEnv(game, seed + i, width=W, height=H) for i in range(n)]
         np.testing.assert_array_equal(sim.reset(), np.stack([r.reset() for r in refs]))
         rs = np.random.RandomState(3)
         for t in range(24):
@@ -165,14 +150,11 @@ def test_human_render_live_oracle(game, oracle_available):
 
 
 @pytest.mark.parametrize("game,mode", [("maze", 2), ("chaser", 2), ("jumper", 2), ("caveflyer", 0)])
-def test_human_render_in_other_modes_live_oracle(game, mode, oracle_available):
+def test_human_render_in_other_modes_live_oracle(game, mode, reference):
     """cenv_render of the instantiations with their own world size (zoom, sprite count and tile window differ)."""
-    if not oracle_available:
-        pytest.skip("oracle/_ref not built")
-    from oracle import ref_env
     n, seed, W, H = 2, 91, 128, 128
     sim = SimAdapter(game, n, seed, distribution_mode=mode)
-    refs = [ref_env.RefEnv(game, seed + i, width=W, height=H, mode=mode) for i in range(n)]
+    refs = [reference.RefEnv(game, seed + i, width=W, height=H, mode=mode) for i in range(n)]
     np.testing.assert_array_equal(sim.reset(), np.stack([r.reset() for r in refs]))
     rs = np.random.RandomState(4)
     for t in range(60):
@@ -189,19 +171,16 @@ def test_human_render_in_other_modes_live_oracle(game, mode, oracle_available):
 
 
 @pytest.mark.parametrize("game", ["climber", "coinrun", "bossfight"])
-def test_easy_distribution_mode_live_oracle(game, oracle_available):
+def test_easy_distribution_mode_live_oracle(game, reference):
     """Make-option distribution_mode = 0 (easy) against the reference with its compile-time Config::easy_mode flipped
     (climber: enemy probability .2 instead of .5, tilemap.cpp:118; coinrun: the flag only feeds a variable nothing reads,
     tilemap.cpp:148 — same levels as hard; bossfight: System_Mob_AI::Config::mode, boss bullets at half speed and shielded
     phases of 180 + 30 u instead of 180 + 80 u steps, common_systems.cpp:104, 202)."""
-    if not oracle_available:
-        pytest.skip("oracle/_ref not built")
-    from oracle import ref_env
     n, seed, T, ep = (6, 9100, 120, 30) if game != "bossfight" else (4, 9100, 700, 350)
     rs = np.random.RandomState(12)
     acts = rs.randint(0, 15, size=(T, n)).astype(np.int32)
     sim = SimAdapter(game, n, seed, max_episode_steps=ep, distribution_mode=0)
-    refs = [ref_env.RefEnv(game, seed + i, **(dict(mode=0) if game == "bossfight" else dict(easy_mode=True))) for i in range(n)]
+    refs = [reference.RefEnv(game, seed + i, **(dict(mode=0) if game == "bossfight" else dict(easy_mode=True))) for i in range(n)]
     np.testing.assert_array_equal(sim.reset(), np.stack([r.reset() for r in refs]))
     age = np.zeros(n, np.int64)
     for t in range(T):
@@ -229,17 +208,14 @@ def test_easy_distribution_mode_live_oracle(game, oracle_available):
 
 
 @pytest.mark.parametrize("game,mode", [("maze", 0), ("maze", 2), ("chaser", 1), ("chaser", 2), ("jumper", 0), ("caveflyer", 0), ("jumper", 2), ("caveflyer", 2)])
-def test_world_size_modes_live_oracle(game, mode, oracle_available):
+def test_world_size_modes_live_oracle(game, mode, reference):
     """Distribution modes that change the world size (own instantiations, G = <Game>T<MODE>) against the reference with its
     compile-time Config::mode set through the probe: levels (tile map + RNG state), pixels, rewards, dones, truncation."""
-    if not oracle_available:
-        pytest.skip("oracle/_ref not built")
-    from oracle import ref_env
     n, seed, T = 5, 8300 + mode, 150
     rs = np.random.RandomState(mode)
     acts = rs.randint(0, 15, size=(T, n)).astype(np.int32)
     sim = SimAdapter(game, n, seed, max_episode_steps=40, distribution_mode=mode)
-    refs = [ref_env.RefEnv(game, seed + i, mode=mode) for i in range(n)]
+    refs = [reference.RefEnv(game, seed + i, mode=mode) for i in range(n)]
     f = sim.fields()
     for i, r in enumerate(refs):   # level #1 (cenv_make)
         rt = r.tiles()
@@ -292,17 +268,14 @@ def bossfight_policy(read_field, n, rs):
 
 
 @pytest.mark.parametrize("mode", [None, 0])
-def test_bossfight_whole_fight_live_oracle(mode, oracle_available):
+def test_bossfight_whole_fight_live_oracle(mode, reference):
     """bossfight beyond the first seconds (System_Mob_AI::update common_systems.cpp:199-390: shielded / unshielded phases,
     every attack pattern, hp, the boss's death and the win reward) with a policy that survives: pixels, rewards, dones every
     step, RNG state at the end, hard and easy mode."""
-    if not oracle_available:
-        pytest.skip("oracle/_ref not built")
-    from oracle import ref_env
     n, seed, T = 8, 777, 1500
     rs = np.random.RandomState(seed)
     sim = SimAdapter("bossfight", n, seed, distribution_mode=-1 if mode is None else mode)
-    refs = [ref_env.RefEnv("bossfight", seed + i, mode=mode) for i in range(n)]
+    refs = [reference.RefEnv("bossfight", seed + i, mode=mode) for i in range(n)]
     np.testing.assert_array_equal(sim.reset(), np.stack([r.reset() for r in refs]))
     wins, longest, age = 0, 0, np.zeros(n, np.int64)
     for t in range(T):
@@ -327,17 +300,14 @@ def test_bossfight_whole_fight_live_oracle(mode, oracle_available):
 
 
 @pytest.mark.parametrize("mode", [None, 2])
-def test_chaser_orbs_and_eaten_mobs_live_oracle(mode, oracle_available):
+def test_chaser_orbs_and_eaten_mobs_live_oracle(mode, reference):
     """chaser with a corridor-walking policy (hold a direction, turn now and then): the agent covers the maze, eats orbs
     (System_Mob_AI::eat, mobs flee and slow down, common_systems.cpp:117-297) and, now and then, a mob (respawn as an egg on
     a free cell drawn from the RNG, y not flipped: SURVEY Q17) — paths uniform-random actions hardly reach."""
-    if not oracle_available:
-        pytest.skip("oracle/_ref not built")
-    from oracle import ref_env
     n, seed, T = 16, 555, 1500
     rs = np.random.RandomState(seed)
     sim = SimAdapter("chaser", n, seed, distribution_mode=-1 if mode is None else mode)
-    refs = [ref_env.RefEnv("chaser", seed + i, mode=mode) for i in range(n)]
+    refs = [reference.RefEnv("chaser", seed + i, mode=mode) for i in range(n)]
     np.testing.assert_array_equal(sim.reset(), np.stack([r.reset() for r in refs]))
     cur = rs.choice([1, 7, 3, 5], size=n)
     orbs, prev_eat = 0, np.zeros(n, np.float32)
