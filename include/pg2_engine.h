@@ -65,7 +65,10 @@ PG2_API int32_t pg2_step_device(pg2_engine* e, const int32_t* actions_device);
 
 /* cenv_render (games/coinrun/coinrun.cpp:393-411): environment `env`'s current scene drawn again at width x height with the
  * window size as camera_size (render_game(false): camera_scale = game_zoom * width / 64), as width * height * 3 RGB
- * bytes (row-major) in HOST memory. A cold path for the human viewer; synchronous. */
+ * bytes (row-major) in HOST memory. A cold path for the human viewer; synchronous.
+ * Fails (nonzero, pg2_last_error) rather than return an incomplete frame when width or height exceeds 32767 pixels (blit
+ * rects are 16-bit pixel coordinates) or when the window spans more tile rows than the game's frame tables hold
+ * (WIN_ROWS: a window much taller than wide; e.g. maze at 64 x 4096). */
 PG2_API int32_t pg2_render_human(pg2_engine* e, int32_t env, int32_t width, int32_t height, uint8_t* out_rgb);
 
 /* Copy results of the last step/reset to host buffers (any pointer may be NULL) and wait.

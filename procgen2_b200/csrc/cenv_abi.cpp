@@ -49,7 +49,7 @@ std::vector<pg2_engine*> g_engines;
 std::vector<int> g_first, g_count;
 pg2_engine* g_engine = nullptr;   // == g_engines[0] (non-null <=> made)
 int g_num_envs = 1;
-int g_window_w = 512, g_window_h = 512;
+int g_window_w = 512, g_window_h = 512;   // cenv_render's window (options "width" / "height"; limits: pg2_render_human)
 
 int g_host_copy = 1;              // make-option "host_copy": 0 = observations stay in HBM (read them through the device pointers)
 

@@ -66,21 +66,6 @@ __global__ void k_seed(CommonState c, int N, uint32_t base_seed, const int32_t* 
     seed_body(c, env, seeds ? (uint32_t)seeds[env] : base_seed + (uint32_t)env, init_persistent != 0);
 }
 
-// Level prefetch (G::PREFETCH_LEVELS): the NEXT level of every env is generated one episode ahead into a shadow copy of the
-// state (k_reset on the shadow state, asynchronous, second stream). When an env finishes, k_step makes sure that level exists
-// (swap_wait) and flags the env in `pending`; the render CTA that draws the env copies the shadow's reset-written fields over
-// the live ones first (swap_copy), and the env goes onto the generator's list, which prepares the level after that. Field
-// table: one entry per copied SoA field.
-struct SwapField { char* live; const char* shadow; int esz, per_env, env_major; };
-constexpr int MAX_SWAP_FIELDS = 64;
-struct SwapTable { SwapField f[MAX_SWAP_FIELDS]; int n; };
-struct SwapArgs {
-    SwapTable table;          // table.n == 0: no level prefetch
-    CommonState shadow_c;
-    const int* gen_done;      // [N] levels delivered by the generator (beyond the first)
-    int* used;                // [N] levels taken
-};
-
 // k_step, lane 0 of the warp / lane group that finished an env: wait until the generator has delivered the level this env is
 // about to take (ready <=> gen_done >= used; almost always true on arrival — the generator had a whole episode; the poll is
 // bounded so that a logic error can never hang the GPU: fault bit 4 instead). The wait sits in k_step, whose CTAs come and
@@ -92,68 +77,6 @@ __device__ __forceinline__ void swap_wait(const SwapArgs& a, const CommonState& 
     while (*g < need && spins < (1 << 18)) { __nanosleep(200); spins++; }
     if (*g < need) live_c.fault[env] |= 4;
     __threadfence();
-}
-
-// k_render, the whole CTA that is about to draw a finished env: copy the reset-written fields shadow -> live. Loads are issued
-// in batches before their stores (the compiler cannot prove that a store does not alias the next load, which would
-// serialise one memory round trip per element): short fields (<= blockDim elements per env) eight fields per round, one
-// element per thread; long ones (tile map, MT19937 words, particle pools) eight elements per thread per round.
-__device__ __noinline__ void swap_copy(const SwapArgs& a, const CommonState& live_c, int env, int N) {
-    const int tid = threadIdx.x, nthr = CTA_THREADS;   // called by the render CTA
-    __threadfence();
-    auto elem_off = [&](const SwapField& f, int j) { return f.env_major ? ((size_t)env * f.per_env + j) * f.esz : ((size_t)j * N + env) * f.esz; };
-    for (int i0 = 0; i0 < a.table.n; i0 += 8) {
-        uint32_t v[8];
-#pragma unroll
-        for (int k = 0; k < 8; k++) {
-            v[k] = 0u;
-            if (i0 + k >= a.table.n) continue;
-            const SwapField f = a.table.f[i0 + k];
-            if (f.per_env > nthr || tid >= f.per_env || (f.esz != 4 && f.esz != 1)) continue;
-            const size_t off = elem_off(f, tid);
-            v[k] = f.esz == 4 ? *(const uint32_t*)(f.shadow + off) : (uint32_t)(uint8_t)f.shadow[off];
-        }
-#pragma unroll
-        for (int k = 0; k < 8; k++) {
-            if (i0 + k >= a.table.n) continue;
-            const SwapField f = a.table.f[i0 + k];
-            if (f.per_env > nthr || tid >= f.per_env || (f.esz != 4 && f.esz != 1)) continue;
-            const size_t off = elem_off(f, tid);
-            if (f.esz == 4) *(uint32_t*)(f.live + off) = v[k]; else f.live[off] = (char)v[k];
-        }
-    }
-    for (int i = 0; i < a.table.n; i++) {
-        const SwapField f = a.table.f[i];
-        if (f.per_env <= nthr && (f.esz == 4 || f.esz == 1)) continue;
-        if (f.esz != 4 && f.esz != 1) {   // odd element sizes (none today)
-            for (int j = tid; j < f.per_env; j += nthr) { const size_t off = elem_off(f, j); for (int bb = 0; bb < f.esz; bb++) f.live[off + bb] = f.shadow[off + bb]; }
-            continue;
-        }
-        // an env-major byte field whose per-env block is word-aligned is copied as words
-        const bool as_words = f.env_major && f.esz == 1 && ((((size_t)env * f.per_env) | (size_t)f.per_env | (size_t)(uintptr_t)f.live | (size_t)(uintptr_t)f.shadow) & 3) == 0;
-        const int count = as_words ? f.per_env / 4 : f.per_env, esz = as_words ? 4 : f.esz;
-        for (int j0 = 0; j0 < count; j0 += 8 * nthr) {
-            uint32_t u[8];
-#pragma unroll
-            for (int q = 0; q < 8; q++) {
-                const int j = j0 + q * nthr + tid;
-                const size_t off = f.env_major ? ((size_t)env * f.per_env * f.esz + (size_t)j * esz) : ((size_t)j * N + env) * esz;
-                u[q] = j >= count ? 0u : esz == 4 ? *(const uint32_t*)(f.shadow + off) : (uint32_t)(uint8_t)f.shadow[off];
-            }
-#pragma unroll
-            for (int q = 0; q < 8; q++) {
-                const int j = j0 + q * nthr + tid;
-                const size_t off = f.env_major ? ((size_t)env * f.per_env * f.esz + (size_t)j * esz) : ((size_t)j * N + env) * esz;
-                if (j < count) { if (esz == 4) *(uint32_t*)(f.live + off) = u[q]; else f.live[off] = (char)u[q]; }
-            }
-        }
-    }
-    if (tid == 0) {   // what reset_body does besides the level
-        a.used[env] += 1;   // read by this env's next wait only
-        live_c.ep_steps[env] = 0; live_c.view_valid[env] = 0;
-        live_c.fault[env] |= a.shadow_c.fault[env];
-    }
-    __syncthreads();   // the CTA reads what it just wrote
 }
 
 // Finished envs are appended to `list` (ballot + one atomic per warp on *count) and flagged in `pending` (an overlapped
@@ -227,75 +150,6 @@ __global__ void __launch_bounds__(32 * RESET_WARPS_PER_CTA) k_reset(typename G::
             if (lane == 0) atomicAdd(&gen_done[env], 1);
         }
     }
-}
-
-// Persistent CTAs; frames are handed out through a ticket counter, so a CTA that drew cheap frames simply takes
-// more of them. mode 0: every env; mode 1: every env that is NOT being reset this step (k_reset runs concurrently
-// on a second stream); mode 2: exactly the envs of the reset list (after k_reset).
-template <class G>
-__global__ void __launch_bounds__(RENDER_THREADS, G::RENDER_MIN_CTAS) k_render(typename G::State s, CommonState c, const TexInfo* __restrict__ tex,
-                                                           const uint32_t* __restrict__ atlas, uint8_t* __restrict__ obs,
-                                                           int* __restrict__ ticket, int mode, const int* __restrict__ list,
-                                                           const int* __restrict__ list_count, const uint8_t* __restrict__ pending, int N,
-                                                           uint8_t* __restrict__ view_cache, const __grid_constant__ SwapArgs swap) {
-    __shared__ FrameOf<G> f;
-    __shared__ int s_env;
-    const int count = mode == 2 ? *list_count : N;
-    frame_init_tiletex<G>(f, tex);
-    // thread 0: the next frame's env (-1: none left) and whether its cached base image is valid — both fetched one frame
-    // ahead, so that their memory round trips overlap the current frame's work (an env's view_valid only changes when the
-    // env itself is rendered, or in earlier kernels)
-    __shared__ int s_swap;
-    int next_env = -1;
-    bool next_reuse = false, next_swap = false;
-    // level prefetch: the envs that finished in this step (the list k_step appended them to) come first — their CTAs copy the
-    // next level in before drawing, which must not land in the kernel's tail — then every env that is not on the list
-    const int nfirst = (swap.table.n > 0 && mode == 0) ? *list_count : 0;
-    auto take_ticket = [&]() {
-        int t = atomicAdd(ticket, 1);
-        if (nfirst > 0) {
-            if (t < nfirst) { next_env = list[t]; next_swap = true; next_reuse = false; return; }
-            t -= nfirst;
-            while (t < count && pending[t]) t = atomicAdd(ticket, 1) - nfirst;
-        }
-        if (mode == 1) while (t < count && pending[t]) t = atomicAdd(ticket, 1);
-        next_env = t < count ? (mode == 2 ? list[t] : t) : -1;
-        next_swap = false;
-        next_reuse = G::STATIC_VIEW && view_cache != nullptr && next_env >= 0 && !next_swap && c.view_valid[next_env] != 0;
-    };
-    if (threadIdx.x == 0) take_ticket();
-    for (;;) {
-#ifdef PG2_PHASE_TIMERS
-        long long phase_t__ = clock64();
-#endif
-        __syncthreads();   // every warp is done with the previous frame (bands are stored per warp, without a CTA barrier)
-        if (threadIdx.x == 0) { s_env = next_env; s_swap = next_swap ? 1 : 0; }
-        frame_begin(f, next_reuse);
-        __syncthreads();
-        const int env = s_env;
-        if (env < 0) break;
-        PG2_PHASE_MARK(1);
-#ifdef PG2_PHASE_TIMERS
-        if (threadIdx.x == 0) atomicAdd(&g_phase[0], 1ull);
-#endif
-        // the next frame's ticket is taken now: the atomic's round trip overlaps this frame's work
-        const bool do_swap = s_swap != 0;
-        if (threadIdx.x == 0) take_ticket();
-        if (do_swap) swap_copy(swap, c, env, N);
-        render_body<G>(s, c, env, f, tex, atlas, obs, view_cache, false);
-    }
-    if ((threadIdx.x & 31) == 0) frame_store_wait();   // every warp issued bulk stores of its own
-}
-
-// Human-mode frame of one env (cenv_render): every CTA shades a contiguous slice of the width x height frame.
-template <class G>
-__global__ void __launch_bounds__(RENDER_THREADS) k_render_human(typename G::State s, CommonState c, int env, const TexInfo* __restrict__ tex,
-                                                                 const uint32_t* __restrict__ atlas, uint8_t* __restrict__ out, int width, int height) {
-    __shared__ FrameOf<G> f;
-    frame_init_tiletex<G>(f, tex);
-    const int total = width * height, per = (total + gridDim.x - 1) / gridDim.x;
-    const int first = blockIdx.x * per, last = min(total, first + per);
-    render_human_body<G>(s, c, env, f, tex, atlas, out, width, height, first, last);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -790,18 +644,27 @@ struct Engine : EngineBase {
     }
 
     // cenv_render: the env's scene at window resolution (render_game(false)), copied to host memory
+    // Blit rects are int16 pixel coordinates (FastBlit), hence at most 32767 pixels per side.
     int render_human(int env, int width, int height, uint8_t* out_host) override {
-        if (env < 0 || env >= N || width < 1 || height < 1 || (long long)width * height > (1 << 26)) return fail("pg2_render_human: bad arguments");
+        if (env < 0 || env >= N || width < 1 || height < 1 || width > 32767 || height > 32767 || (long long)width * height > (1 << 26))
+            return fail("pg2_render_human: bad arguments");
         const size_t bytes = (size_t)width * height * 3;
         uint8_t* dev = nullptr;
-        PG2_CUDA(cudaMalloc(&dev, bytes));
+        PG2_CUDA(cudaMalloc(&dev, bytes + 8));
+        int* dev_overflow = (int*)(dev + ((bytes + 3) & ~(size_t)3));
         const int grid = std::max(1, std::min(num_sms * 2, (width * height + 1023) / 1024));
-        k_render_human<G><<<grid, RENDER_THREADS, 0, stream>>>(st, common, env, texinfo, atlas, dev, width, height);
-        launches++;
-        cudaError_t ce = cudaMemcpyAsync(out_host, dev, bytes, cudaMemcpyDeviceToHost, stream);
+        int overflow = 0;
+        cudaError_t ce = cudaMemsetAsync(dev_overflow, 0, sizeof(int), stream);
+        if (ce == cudaSuccess) {
+            k_render_human<G><<<grid, RENDER_THREADS, 0, stream>>>(st, common, env, texinfo, atlas, dev, width, height, dev_overflow);
+            launches++;
+            ce = cudaMemcpyAsync(out_host, dev, bytes, cudaMemcpyDeviceToHost, stream);
+        }
+        if (ce == cudaSuccess) ce = cudaMemcpyAsync(&overflow, dev_overflow, sizeof(int), cudaMemcpyDeviceToHost, stream);
         if (ce == cudaSuccess) ce = cudaStreamSynchronize(stream);
         cudaFree(dev);
         if (ce != cudaSuccess) return fail(std::string("pg2_render_human: ") + cudaGetErrorString(ce));
+        if (overflow) return fail("pg2_render_human: the window spans more tile rows than the frame tables hold; use a wider aspect ratio");
         return 0;
     }
 

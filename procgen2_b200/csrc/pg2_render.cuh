@@ -63,12 +63,19 @@ struct BlitRot {
 // Per-pixel form of a blit (what the frame keeps): coverage test = two unsigned compares, sampling = one
 // multiply-add + shift per axis (a horizontal flip is folded into hx / incx, which wrap modulo 2^32 to the
 // exact non-negative value), texel address = base + sy * tex_w + sx.
+// A rotated blit is mapped about the centre of its WHOLE integer rect, which can be of any size: it keeps the rect in
+// 32-bit fields instead (rw / rh, and the origin in hx / hy, whose sample phase is always inc / 2: rotated blits are
+// never flipped or clipped).
 struct alignas(16) FastBlit {
-    int16_t x0, y0; uint16_t w, h;              // integer destination rect (SDL truncates the float rect)
-    uint32_t hx, incx;                          // sx = (hx + i * incx) >> 16
-    uint32_t hy, incy, base;                    // base = tex_offset + s0y * tex_w + s0x
+    union {
+        struct { int16_t x0, y0; uint16_t w, h; };   // un-rotated: integer destination rect (SDL truncates the float rect)
+        struct { uint32_t rw, rh; };                 // rotated: width and height of the rect
+    };
+    uint32_t hx, incx;                          // un-rotated: sx = (hx + i * incx) >> 16; rotated: hx = x0 (int32)
+    uint32_t hy, incy, base;                    // (the same for y); base = tex_offset + s0y * tex_w + s0x
     uint16_t tex_w; uint8_t flags, alpha_mod;   // flags: 1 blend, 2 rotated, 4 invisible
 };
+static_assert(sizeof(FastBlit) == 32, "FastBlit is two 16-byte words");
 
 constexpr int MAX_TILE_TEX = 32;
 
@@ -261,18 +268,39 @@ PG2_DEV void frame_store_wait() {
 #endif
 }
 
-PG2_DEV FastBlit make_fast(const Blit& b) {
+// vw x vh: the target (64 x 64, or the window of a human-mode frame, at most 32767 pixels per side). An un-rotated rect
+// outside the 16-bit fields (never one of a game's observation frames) is clipped to the target first, the skipped
+// destination pixels folded into hx / hy (the samples wrap modulo 2^32 exactly like the unclipped ones), so that a rect
+// of any size draws what the spec draws. A rotated rect is kept whole in 32-bit fields (see FastBlit).
+PG2_DEV FastBlit make_fast(const Blit& b, int vw, int vh) {
     FastBlit fb;
-    bool off = b.ax.d0 < -32768 || b.ax.d0 > 32767 || b.ay.d0 < -32768 || b.ay.d0 > 32767 || b.ax.dlen > 65535 || b.ay.dlen > 65535;
-    fb.x0 = (int16_t)b.ax.d0; fb.y0 = (int16_t)b.ay.d0;
-    fb.w = (uint16_t)max(0, b.ax.dlen); fb.h = (uint16_t)max(0, b.ay.dlen);
+    bool off = false;
     fb.incx = b.flip_h ? 0u - b.ax.inc : b.ax.inc;
-    fb.hx = b.flip_h ? b.ax.inc / 2u + (uint32_t)(b.ax.dlen - 1) * b.ax.inc : b.ax.inc / 2u;
-    fb.hy = b.ay.inc / 2u; fb.incy = b.ay.inc;
+    fb.incy = b.ay.inc;
+    if (b.rotated) {
+        fb.rw = (uint32_t)max(0, b.ax.dlen); fb.rh = (uint32_t)max(0, b.ay.dlen);
+        fb.hx = (uint32_t)b.ax.d0; fb.hy = (uint32_t)b.ay.d0;
+    } else {
+        off = b.ax.d0 < -32768 || b.ax.d0 > 32767 || b.ay.d0 < -32768 || b.ay.d0 > 32767 || b.ax.dlen > 65535 || b.ay.dlen > 65535;
+        fb.x0 = (int16_t)b.ax.d0; fb.y0 = (int16_t)b.ay.d0;
+        fb.w = (uint16_t)max(0, b.ax.dlen); fb.h = (uint16_t)max(0, b.ay.dlen);
+        fb.hx = b.flip_h ? b.ax.inc / 2u + (uint32_t)(b.ax.dlen - 1) * b.ax.inc : b.ax.inc / 2u;
+        fb.hy = b.ay.inc / 2u;
+    }
+    if (__builtin_expect(off && b.ax.visible, 0)) {
+        // skip k = -d0 pixels of a rect that starts left of / above the target, keep at most what reaches its far edge
+        const uint32_t kx = b.ax.d0 < 0 ? 0u - (uint32_t)b.ax.d0 : 0u, ky = b.ay.d0 < 0 ? 0u - (uint32_t)b.ay.d0 : 0u;
+        const int x0 = b.ax.d0 < 0 ? 0 : b.ax.d0, y0 = b.ay.d0 < 0 ? 0 : b.ay.d0;
+        const int w = kx >= (uint32_t)b.ax.dlen || x0 >= vw ? 0 : min(b.ax.dlen - (int)kx, vw - x0);
+        const int h = ky >= (uint32_t)b.ay.dlen || y0 >= vh ? 0 : min(b.ay.dlen - (int)ky, vh - y0);
+        off = w == 0 || h == 0;
+        fb.x0 = (int16_t)x0; fb.y0 = (int16_t)y0; fb.w = (uint16_t)w; fb.h = (uint16_t)h;
+        fb.hx = b.flip_h ? fb.hx - kx * b.ax.inc : fb.hx + kx * b.ax.inc;
+        fb.hy += ky * b.ay.inc;
+    }
     fb.base = b.tex_offset + (uint32_t)b.ay.s0 * b.tex_w + (uint32_t)b.ax.s0;
     fb.tex_w = b.tex_w;
     fb.alpha_mod = b.alpha_mod;
-    // a destination rect outside the int16 range cannot intersect the 64x64 target
     fb.flags = (uint8_t)((b.blend ? 1 : 0) | (b.rotated ? 2 : 0) | ((b.ax.visible && !off) ? 0 : 4));
     return fb;
 }
@@ -283,12 +311,12 @@ PG2_DEV FastBlit make_fast(const Blit& b) {
 // the rounding of the test's own arithmetic: a bound only has to be conservative, it never changes which pixels are drawn
 // (bullets a few pixels long got 9-11 px boxes from the integer centre +- (ceil + 2) of round 1: three times the patches).
 PG2_DEV void rotated_bounds(const FastBlit& fb, BlitRot* rot) {
-    const double hw = 0.5 * (double)fb.w, hh = 0.5 * (double)fb.h, ac = fabs(rot->c), as = fabs(rot->s);
+    const double hw = 0.5 * (double)fb.rw, hh = 0.5 * (double)fb.rh, ac = fabs(rot->c), as = fabs(rot->s);
     const double ex = hw * ac + hh * as + 1e-3, ey = hw * as + hh * ac + 1e-3;
-    const double cx = (double)fb.x0 + hw - 0.5, cy = (double)fb.y0 + hh - 0.5;   // pixel index X = centre coordinate - 0.5
+    const double cx = (double)(int32_t)fb.hx + hw - 0.5, cy = (double)(int32_t)fb.hy + hh - 0.5;   // pixel index X = centre coordinate - 0.5
     const double lo_x = floor(cx - ex), hi_x = ceil(cx + ex), lo_y = floor(cy - ey), hi_y = ceil(cy + ey);
-    rot->x_lo = (int16_t)fmax(lo_x, -30000.0); rot->x_hi = (int16_t)fmin(hi_x, 30000.0);
-    rot->y_lo = (int16_t)fmax(lo_y, -30000.0); rot->y_hi = (int16_t)fmin(hi_y, 30000.0);
+    rot->x_lo = (int16_t)fmax(lo_x, -32768.0); rot->x_hi = (int16_t)fmin(hi_x, 32767.0);
+    rot->y_lo = (int16_t)fmax(lo_y, -32768.0); rot->y_hi = (int16_t)fmin(hi_y, 32767.0);
 }
 
 // Bands (8 rows each) a blit can touch.
@@ -342,7 +370,7 @@ PG2_DEV void emit_post_blits(F& f, const TexInfo* tex, int ncand, MakeFn make) {
         else if (req.mode == 3) b = make_blit_rect(tex, req.tex_id, req.x, req.y, req.w, req.h, req.angle_deg, &rot);
         bool vis = req.mode != 0 && b.ax.visible;
         FastBlit fb;
-        if (vis) { fb = make_fast(b); vis = !(fb.flags & 4u); }
+        if (vis) { fb = make_fast(b, (int)f.view_w, (int)f.view_h); vis = !(fb.flags & 4u); }
         uint32_t m = __ballot_sync(0xffffffffu, vis);
         if (lane == 0) f.wcount[round][warp] = __popc(m);
         __syncthreads();
@@ -547,7 +575,7 @@ PG2_DEV_NOINLINE void frame_finalize(F& f) {
     for (int k = tid; k < npre; k += CTA_THREADS) {
         Blit b = f.pre[k];
         if (!b.ay.visible) b.ax.visible = 0;   // make_blit's rule (the two axes were built by different threads)
-        f.fpre[k] = make_fast(b);
+        f.fpre[k] = make_fast(b, (int)f.view_w, (int)f.view_h);
     }
     if (f.human) {   // window-size frame: no 64-pixel tables, every pixel goes the general ordered way
         if (tid == 0) f.wide = 1;
@@ -676,14 +704,15 @@ PG2_DEV bool rotated_texel_coords(int x0, int y0, int w, int h, double rs, doubl
 // Texel of a blit under pixel (X, Y); false when the pixel is not covered.
 template <bool ROT>
 PG2_DEV bool fast_texel(const FastBlit& fb, const BlitRot* rot, const uint32_t* __restrict__ atlas, int X, int Y, uint32_t* texel) {
-    uint32_t i, j;
+    uint32_t i, j, hx = fb.hx, hy = fb.hy;
     if (ROT && (fb.flags & 2u)) {
-        if (!rotated_texel_coords(fb.x0, fb.y0, fb.w, fb.h, rot->s, rot->c, X, Y, &i, &j)) return false;
+        if (!rotated_texel_coords((int32_t)fb.hx, (int32_t)fb.hy, (int)fb.rw, (int)fb.rh, rot->s, rot->c, X, Y, &i, &j)) return false;
+        hx = fb.incx / 2u; hy = fb.incy / 2u;
     } else {
         i = (uint32_t)(X - fb.x0); j = (uint32_t)(Y - fb.y0);
         if (i >= fb.w || j >= fb.h) return false;
     }
-    uint32_t sx = (fb.hx + i * fb.incx) >> 16, sy = (fb.hy + j * fb.incy) >> 16;
+    uint32_t sx = (hx + i * fb.incx) >> 16, sy = (hy + j * fb.incy) >> 16;
     *texel = __ldg(atlas + fb.base + sy * fb.tex_w + sx);
     return true;
 }

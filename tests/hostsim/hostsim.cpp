@@ -28,7 +28,7 @@ struct SimBase {
     virtual void reset_all(const int32_t* seeds) = 0;
     virtual void step(const int32_t* actions) = 0;
     virtual bool find_field(const char* name, void** ptr, int* esz, int* pe) = 0;
-    virtual void render_human(int env, int width, int height, uint8_t* out) = 0;
+    virtual bool render_human(int env, int width, int height, uint8_t* out) = 0;
     int N = 0, max_episode_steps = 0;
     std::vector<uint8_t> obs, terminated, truncated;
     std::vector<float> reward;
@@ -95,8 +95,8 @@ struct Sim : SimBase {
     bool find_field(const char* name, void** ptr, int* esz, int* pe) override {
         return st.find(name, ptr, esz, pe) || c.find(name, ptr, esz, pe);
     }
-    void render_human(int env, int width, int height, uint8_t* out) override {
-        render_human_body<G>(st, c, env, *frame, tex, atlas, out, width, height, 0, width * height);
+    bool render_human(int env, int width, int height, uint8_t* out) override {
+        return render_human_body<G>(st, c, env, *frame, tex, atlas, out, width, height, 0, width * height);
     }
 };
 
@@ -130,7 +130,8 @@ void* hs_create_mode(const char* game, int n, int seed, int max_ep, const char* 
 void hs_destroy(void* h) { delete (SimBase*)h; }
 void hs_reset(void* h, const int32_t* seeds) { ((SimBase*)h)->reset_all(seeds); }
 void hs_step(void* h, const int32_t* actions) { ((SimBase*)h)->step(actions); }
-void hs_render_human(void* h, int env, int width, int height, uint8_t* out) { ((SimBase*)h)->render_human(env, width, height, out); }
+// 0: done; 1: the window spans more tile rows than the frame tables hold (the engine's pg2_render_human fails)
+int hs_render_human(void* h, int env, int width, int height, uint8_t* out) { return ((SimBase*)h)->render_human(env, width, height, out) ? 0 : 1; }
 const uint8_t* hs_obs(void* h) { return ((SimBase*)h)->obs.data(); }
 const float* hs_reward(void* h) { return ((SimBase*)h)->reward.data(); }
 const uint8_t* hs_terminated(void* h) { return ((SimBase*)h)->terminated.data(); }

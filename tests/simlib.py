@@ -63,7 +63,8 @@ class HostSim:
 
     def render_human(self, env, width, height):
         out = np.empty((height, width, 3), np.uint8)
-        lib().hs_render_human(self.h, env, width, height, out.ctypes.data)
+        if lib().hs_render_human(self.h, env, width, height, out.ctypes.data):
+            raise RuntimeError("render_human: the %dx%d window spans more tile rows than the frame tables hold" % (width, height))
         return out
 
     def field(self, name):
