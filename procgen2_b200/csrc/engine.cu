@@ -184,8 +184,8 @@ struct EngineBase {
     virtual size_t state_bytes_per_env() = 0;
     virtual size_t state_alloc_bytes() = 0;     // bytes of state_mem
     virtual uint32_t game_tag() = 0;
-    virtual int init_shadow() = 0;
-    virtual int destroy_graphs() = 0;           // the captured step graphs (they hold pointers into this engine's buffers)              // level prefetch: regenerate every env's next level (after state was written)
+    virtual int init_shadow() = 0;              // level prefetch: regenerate every env's next level (after state was written)
+    virtual int destroy_graphs() = 0;           // the captured step graphs (they hold pointers into this engine's buffers)
 
     int device = 0, N = 0, max_episode_steps = 0, auto_reset = 1;
     uint32_t base_seed = 0;
@@ -198,10 +198,11 @@ struct EngineBase {
     void* state_mem = nullptr;
     void* common_mem = nullptr;
     CommonState common;
-    uint8_t* obs = nullptr;
-    float* reward = nullptr;
-    uint8_t* terminated = nullptr;
-    uint8_t* truncated = nullptr;
+    // The results of a step. Set 0 is allocated by init and is the only one until pipelined stepping starts; then the
+    // steps alternate between the two sets. out[cur] is the set the last step wrote (and the device pointers expose).
+    struct Outputs { uint8_t* obs = nullptr; float* reward = nullptr; uint8_t* terminated = nullptr; uint8_t* truncated = nullptr; };
+    Outputs out[2];
+    int cur = 0;
     int32_t* actions = nullptr;
     int32_t* seeds_dev = nullptr;
     int* reset_list = nullptr;
@@ -214,13 +215,8 @@ struct EngineBase {
     TexInfo* texinfo = nullptr;
     uint32_t* atlas = nullptr;
     int32_t* actions_pinned = nullptr;
-    // depth-1 pipelined stepping (pg2_step_pipelined): double-buffered outputs + a copy stream
+    // depth-1 pipelined stepping (pg2_step_pipelined): output set 1 + a copy stream
     bool pipelined = false;
-    int cur = 0;
-    uint8_t* obs_b[2] = { nullptr, nullptr };
-    float* reward_b[2] = { nullptr, nullptr };
-    uint8_t* term_b[2] = { nullptr, nullptr };
-    uint8_t* trunc_b[2] = { nullptr, nullptr };
     int32_t* actions_b[2] = { nullptr, nullptr };
     int32_t* pinned_b[2] = { nullptr, nullptr };
     cudaStream_t copy_stream = nullptr;
@@ -282,12 +278,20 @@ struct EngineBase {
         return 0;
     }
 
+    int alloc_outputs(Outputs& o) {
+        PG2_CUDA(cudaMalloc(&o.obs, (size_t)N * OBS_BYTES));
+        PG2_CUDA(cudaMalloc(&o.reward, sizeof(float) * N));
+        PG2_CUDA(cudaMalloc(&o.terminated, N));
+        PG2_CUDA(cudaMalloc(&o.truncated, N));
+        return 0;
+    }
+
     int free_all() {
         DeviceGuard guard(device);
         if (stream) cudaStreamSynchronize(stream);
-        if (pipelined) { cudaStreamSynchronize(copy_stream); obs = obs_b[0]; reward = reward_b[0]; terminated = term_b[0]; truncated = trunc_b[0]; }
-        cudaFree(state_mem); cudaFree(common_mem); cudaFree(obs); cudaFree(reward); cudaFree(terminated);
-        cudaFree(truncated); cudaFree(actions); cudaFree(seeds_dev); cudaFree(reset_list); cudaFree(reset_count); cudaFree(view_cache);
+        if (pipelined) cudaStreamSynchronize(copy_stream);
+        for (Outputs& o : out) { cudaFree(o.obs); cudaFree(o.reward); cudaFree(o.terminated); cudaFree(o.truncated); }
+        cudaFree(state_mem); cudaFree(common_mem); cudaFree(actions); cudaFree(seeds_dev); cudaFree(reset_list); cudaFree(reset_count); cudaFree(view_cache);
         for (int j = 0; j < PREP_SLOTS; j++) if (prep_streams[j]) { cudaStreamSynchronize(prep_streams[j]); cudaStreamDestroy(prep_streams[j]); }
         for (int j = 0; j < PREP_SLOTS; j++) if (ev_prepared[j]) cudaEventDestroy(ev_prepared[j]);
         cudaFree(shadow_state_mem); cudaFree(shadow_common_mem); cudaFree(prep_list); cudaFree(prep_count); cudaFree(gen_done); cudaFree(gen_used);
@@ -297,8 +301,6 @@ struct EngineBase {
         destroy_graphs();
         if (actions_pinned) cudaFreeHost(actions_pinned);
         if (pipelined) {
-            // slot 0 aliases the primary buffers (freed above)
-            cudaFree(obs_b[1]); cudaFree(reward_b[1]); cudaFree(term_b[1]); cudaFree(trunc_b[1]);
             for (int k = 0; k < 2; k++) { cudaFree(actions_b[k]); cudaFreeHost(pinned_b[k]); cudaEventDestroy(ev_step[k]); cudaEventDestroy(ev_copy[k]); cudaEventDestroy(ev_h2d[k]); }
             cudaStreamDestroy(copy_stream);
         }
@@ -320,7 +322,6 @@ struct Engine : EngineBase {
         PG2_CUDA(cudaGetDeviceProperties(&prop, device));
         num_sms = prop.multiProcessorCount;
         PG2_CUDA(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
-        // k_step mapping: aim for >= 8 warps per SM sub-partition before packing several envs into one warp
         // lane-aware games always give a whole warp to an environment; the others pack several environments
         // into a warp once there are >= 8 warps per SM sub-partition
         step_epw = 1;
@@ -336,14 +337,11 @@ struct Engine : EngineBase {
             return fail("pg2_create: distribution_mode " + std::to_string(cfg->distribution_mode) + " is not available for this game "
                         "(0 easy, 1 hard, 2 memory / extreme; built: every game's reference default, + easy for coinrun and climber)");
         common.mode = cfg->distribution_mode;
-        PG2_CUDA(cudaMalloc(&obs, (size_t)N * OBS_BYTES));
-        PG2_CUDA(cudaMemsetAsync(obs, 0, (size_t)N * OBS_BYTES, stream));
-        PG2_CUDA(cudaMalloc(&reward, sizeof(float) * N));
-        PG2_CUDA(cudaMalloc(&terminated, N));
-        PG2_CUDA(cudaMalloc(&truncated, N));
-        PG2_CUDA(cudaMemsetAsync(reward, 0, sizeof(float) * N, stream));
-        PG2_CUDA(cudaMemsetAsync(terminated, 0, N, stream));
-        PG2_CUDA(cudaMemsetAsync(truncated, 0, N, stream));
+        if (alloc_outputs(out[0])) return 1;
+        PG2_CUDA(cudaMemsetAsync(out[0].obs, 0, (size_t)N * OBS_BYTES, stream));
+        PG2_CUDA(cudaMemsetAsync(out[0].reward, 0, sizeof(float) * N, stream));
+        PG2_CUDA(cudaMemsetAsync(out[0].terminated, 0, N, stream));
+        PG2_CUDA(cudaMemsetAsync(out[0].truncated, 0, N, stream));
         PG2_CUDA(cudaMalloc(&actions, sizeof(int32_t) * N));
         PG2_CUDA(cudaMalloc(&seeds_dev, sizeof(int32_t) * N));
         PG2_CUDA(cudaMalloc(&reset_list, sizeof(int) * N));
@@ -405,7 +403,7 @@ struct Engine : EngineBase {
         // cenv_make: seed, then reset() once (level #1 is generated and never rendered, Q29)
         k_seed<<<(N + 127) / 128, 128, 0, stream>>>(common, N, base_seed, nullptr, 1);
         launches++;
-        launch_reset_all();
+        launch_reset(st, common, nullptr, nullptr, nullptr, stream);
         if (init_shadow()) return 1;
         PG2_CUDA(cudaGetLastError());
         PG2_CUDA(cudaStreamSynchronize(stream));
@@ -418,23 +416,22 @@ struct Engine : EngineBase {
         swap_table.n = 0;
         const std::string keeps = G::reset_keeps();
         bool overflow = false;
-        auto add = [&](const char* name, void* live_ptr, void* shadow_ptr, int esz, int per_env) {
+        auto add = [&](const char* name, void* live_ptr, void* shadow_ptr, int esz, int per_env, bool env_major) {
             if (keeps.find(std::string(" ") + name + " ") != std::string::npos) return;
             if (swap_table.n >= MAX_SWAP_FIELDS) { overflow = true; return; }
-            const bool env_major = !strcmp(name, "tiles") || !strcmp(name, "mt");
             swap_table.f[swap_table.n++] = SwapField{ (char*)live_ptr, (const char*)shadow_ptr, esz, per_env, env_major ? 1 : 0 };
         };
         std::vector<void*> shadow_ptrs;
-        shadow_st.for_each_field([&](const char*, void* p, int, int) { shadow_ptrs.push_back(p); });
+        shadow_st.for_each_field([&](const char*, void* p, int, int, bool) { shadow_ptrs.push_back(p); });
         size_t i = 0;
-        st.for_each_field([&](const char* name, void* p, int esz, int pe) { add(name, p, shadow_ptrs[i++], esz, pe); });
+        st.for_each_field([&](const char* name, void* p, int esz, int pe, bool em) { add(name, p, shadow_ptrs[i++], esz, pe, em); });
         std::vector<void*> shadow_cptrs;
-        shadow_common.for_each_field([&](const char*, void* p, int, int) { shadow_cptrs.push_back(p); });
+        shadow_common.for_each_field([&](const char*, void* p, int, int, bool) { shadow_cptrs.push_back(p); });
         i = 0;
-        common.for_each_field([&](const char* name, void* p, int esz, int pe) {
+        common.for_each_field([&](const char* name, void* p, int esz, int pe, bool em) {
             void* sp = shadow_cptrs[i++];
             if (!strcmp(name, "mt") || !strcmp(name, "mti") || !strcmp(name, "sprites_valid") || !strcmp(name, "cam_x") || !strcmp(name, "cam_y"))
-                add(name, p, sp, esz, pe);
+                add(name, p, sp, esz, pe, em);
         });
         if (overflow) return fail("level prefetch: too many state fields for the swap table");
         return 0;
@@ -447,8 +444,7 @@ struct Engine : EngineBase {
         for (int j = 0; j < PREP_SLOTS; j++) PG2_CUDA(cudaStreamSynchronize(prep_streams[j]));
         PG2_CUDA(cudaMemcpyAsync(shadow_state_mem, state_mem, G::State::bytes(N), cudaMemcpyDeviceToDevice, stream));
         PG2_CUDA(cudaMemcpyAsync(shadow_common_mem, common_mem, CommonState::bytes(N), cudaMemcpyDeviceToDevice, stream));
-        k_reset<G><<<reset_grid(N), 32 * RESET_WARPS_PER_CTA, reset_smem(), stream>>>(shadow_st, shadow_common, nullptr, nullptr, N);
-        launches++;
+        launch_reset(shadow_st, shadow_common, nullptr, nullptr, nullptr, stream);
         PG2_CUDA(cudaMemsetAsync(prep_count, 0, PREP_SLOTS * sizeof(int), stream));
         PG2_CUDA(cudaMemsetAsync(gen_done, 0, sizeof(int) * (size_t)N, stream));   // ready <=> gen_done >= used
         PG2_CUDA(cudaMemsetAsync(gen_used, 0, sizeof(int) * (size_t)N, stream));
@@ -471,8 +467,16 @@ struct Engine : EngineBase {
         int ctas = (count + RESET_WARPS_PER_CTA - 1) / RESET_WARPS_PER_CTA;
         return ctas < num_sms * per_sm ? (ctas < 1 ? 1 : ctas) : num_sms * per_sm;
     }
-    void launch_reset_all() {
-        k_reset<G><<<reset_grid(N), 32 * RESET_WARPS_PER_CTA, reset_smem(), stream>>>(st, common, nullptr, nullptr, N);
+    // One helper per kernel of a step; each enqueues its kernel and counts the launch (pg2_kernel_launches).
+    int launch_step(cudaStream_t on) {
+        const cudaKernelNodeParams p = step_node_params();
+        PG2_CUDA(cudaLaunchKernel(p.func, p.gridDim, p.blockDim, p.kernelParams, p.sharedMemBytes, on));
+        launches++;
+        return 0;
+    }
+    // list == nullptr: every env of `s` resets; gen_done: the level generator of the shadow state publishes its levels
+    void launch_reset(const typename G::State& s, const CommonState& c, const int* list, const int* count, int* gen_done, cudaStream_t on) {
+        k_reset<G><<<reset_grid(N), 32 * RESET_WARPS_PER_CTA, reset_smem(), on>>>(s, c, list, count, N, gen_done);
         launches++;
     }
     void launch_render(int mode, int* ticket, cudaStream_t on) {
@@ -481,7 +485,7 @@ struct Engine : EngineBase {
         // (level prefetch: the list / counter k_step appended this step's finished envs to)
         const int* lst = prefetch && ka_list ? ka_list : reset_list;
         const int* cnt = prefetch && ka_count ? ka_count : reset_count + parity;
-        k_render<G><<<grid, RENDER_THREADS, 0, on>>>(st, common, texinfo, atlas, obs, ticket, mode, lst, cnt, pending, N, view_cache, swap_args);
+        k_render<G><<<grid, RENDER_THREADS, 0, on>>>(st, common, texinfo, atlas, out[cur].obs, ticket, mode, lst, cnt, pending, N, view_cache, swap_args);
         launches++;
     }
 
@@ -494,15 +498,15 @@ struct Engine : EngineBase {
             k_seed<<<(N + 127) / 128, 128, 0, stream>>>(common, N, 0u, seeds_dev, 0);
             launches++;
         }
-        launch_reset_all();
+        launch_reset(st, common, nullptr, nullptr, nullptr, stream);
         if (init_shadow()) return 1;
         PG2_CUDA(cudaMemsetAsync(reset_count + 2, 0, 2 * sizeof(int), stream));
         PG2_CUDA(cudaMemsetAsync(pending, 0, N, stream));   // no env of the last step is waiting for its level swap any more
         ka_list = nullptr; ka_count = nullptr;              // ... and the render below has no swap list (reset_count[0..1] stay zero for these games)
         launch_render(0, reset_count + 2, stream);
-        PG2_CUDA(cudaMemsetAsync(reward, 0, sizeof(float) * N, stream));
-        PG2_CUDA(cudaMemsetAsync(terminated, 0, N, stream));
-        PG2_CUDA(cudaMemsetAsync(truncated, 0, N, stream));
+        PG2_CUDA(cudaMemsetAsync(out[cur].reward, 0, sizeof(float) * N, stream));
+        PG2_CUDA(cudaMemsetAsync(out[cur].terminated, 0, N, stream));
+        PG2_CUDA(cudaMemsetAsync(out[cur].truncated, 0, N, stream));
         PG2_CUDA(cudaGetLastError());
         return 0;
     }
@@ -513,16 +517,18 @@ struct Engine : EngineBase {
     // a second stream while the following steps run — up to PREP_SLOTS generator launches in flight, each with a private
     // list (k_step appends to the slot's list directly); an env that finishes again before its next level exists
     // (episodes shorter than a generation) is waited for individually.
-    // The main-stream sequence is captured ONCE per (step parity, list slot, output buffer set) into a CUDA graph and
+    // The main-stream sequence is captured ONCE per (step parity, list slot, output set) into a CUDA graph and
     // replayed: one launch per step; only the pointer to the caller's actions is re-pointed (PG2_GRAPH=0: eager launches).
     // With overlap_reset (PG2_PREFETCH=0 on the slow-generator games) the level generation of the few finished envs runs
     // WHILE a second stream renders all other envs, a short tail render of the reset envs follows (eager only).
-    // Timing marks (pg2_profile, eager): [0] k_step, [1] exposed reset (+ tail render), [2] (main) render.
+    // Timing marks (pg2_profile, eager): [0] k_step, [1] k_reset on the main stream, [2] render (overlap_reset: the
+    // render on the second stream; the wait for it and the tail render are not counted).
     SwapArgs swap_args;             // table.n == 0 when the engine does not prefetch levels
     const int32_t* ka_actions = nullptr;
     int *ka_list = nullptr, *ka_count = nullptr, *ka_zero_a = nullptr, *ka_zero_b = nullptr;
     void* step_kargs[16];
-    struct StepGraph { cudaGraph_t graph = nullptr; cudaGraphExec_t exec = nullptr; cudaGraphNode_t step_node = nullptr; const int32_t* actions = nullptr; uint8_t* obs = nullptr; };
+    struct StepGraph { cudaGraph_t graph = nullptr; cudaGraphExec_t exec = nullptr; cudaGraphNode_t step_node = nullptr; const int32_t* actions = nullptr;
+                       int outputs = -1, kernels = 0; };   // outputs: the output set (out[]) it writes; kernels: its kernel nodes
     StepGraph graphs[2 * PREP_SLOTS];
     bool use_graph = true;
 
@@ -534,7 +540,8 @@ struct Engine : EngineBase {
             ka_list = reset_list; ka_count = reset_count + parity; ka_zero_a = reset_count + (parity ^ 1);
         }
         ka_zero_b = reset_count + 2;
-        void* v[16] = { &st, &common, &ka_actions, &reward, &terminated, &truncated, &ka_list, &ka_count, &pending, &ka_zero_a, &ka_zero_b,
+        Outputs& o = out[cur];
+        void* v[16] = { &st, &common, &ka_actions, &o.reward, &o.terminated, &o.truncated, &ka_list, &ka_count, &pending, &ka_zero_a, &ka_zero_b,
                         &N, &max_episode_steps, &auto_reset, &step_epw, &swap_args };
         memcpy(step_kargs, v, sizeof(v));
     }
@@ -545,18 +552,29 @@ struct Engine : EngineBase {
         p.kernelParams = step_kargs; p.extra = nullptr;
         return p;
     }
-    // the main-stream kernels of one step (eager or under stream capture)
-    int enqueue_main(bool prof) {
+    // The main-stream sequence of one step, eager or under stream capture (not overlap_reset).
+    int enqueue_step(bool prof) {
         if (prof) prof_mark();
-        PG2_CUDA(cudaLaunchKernel((const void*)k_step<G>, dim3(step_grid()), dim3(128), step_kargs, 0, stream));
-        launches++;
+        if (launch_step(stream)) return 1;
         if (prof) prof_mark();
-        if (!prefetch) {
-            k_reset<G><<<reset_grid(N), 32 * RESET_WARPS_PER_CTA, reset_smem(), stream>>>(st, common, reset_list, reset_count + parity, N);
-            launches++;
+        if (overlap_reset) {   // fork: the render of all OTHER envs runs on the second stream
+            PG2_CUDA(cudaEventRecord(ev_stepped, stream));
+            PG2_CUDA(cudaStreamWaitEvent(reset_stream, ev_stepped, 0));
         }
+        // (overlap_reset: k_reset stays on the main stream, first in line after k_step, so that its few long-running CTAs
+        // get their shared memory before the render fills the SMs)
+        if (!prefetch) launch_reset(st, common, reset_list, reset_count + parity, nullptr, stream);
         if (prof) prof_mark();
-        launch_render(0, reset_count + 2, stream);
+        if (overlap_reset) {
+            if (prof) prof_mark_on(reset_stream);
+            launch_render(1, reset_count + 2, reset_stream);
+            if (prof) prof_mark_on(reset_stream);
+            PG2_CUDA(cudaEventRecord(ev_reset_done, reset_stream));   // = main render done
+            PG2_CUDA(cudaStreamWaitEvent(stream, ev_reset_done, 0));
+            launch_render(2, reset_count + 3, stream);
+        } else {
+            launch_render(0, reset_count + 2, stream);
+        }
         if (prof) prof_mark();
         return 0;
     }
@@ -577,37 +595,17 @@ struct Engine : EngineBase {
             PG2_CUDA(cudaStreamWaitEvent(stream, ev_prepared[(slot + 1) % PREP_SLOTS], 0));
         }
         bind_step_args(actions_dev, slot);
-        if (overlap_reset) {
-            // k_reset stays on the main stream (first in line after k_step, so its few long-running CTAs get their
-            // shared memory before the render fills the SMs); the render of all OTHER envs runs on the second stream
-            if (prof) prof_mark();
-            PG2_CUDA(cudaLaunchKernel((const void*)k_step<G>, dim3(step_grid()), dim3(128), step_kargs, 0, stream));
-            launches++;
-            if (prof) prof_mark();
-            PG2_CUDA(cudaEventRecord(ev_stepped, stream));
-            PG2_CUDA(cudaStreamWaitEvent(reset_stream, ev_stepped, 0));
-            k_reset<G><<<reset_grid(N), 32 * RESET_WARPS_PER_CTA, reset_smem(), stream>>>(st, common, reset_list, reset_count + parity, N);
-            if (prof) prof_mark();
-            if (prof) prof_mark_on(reset_stream);
-            launch_render(1, reset_count + 2, reset_stream);
-            if (prof) prof_mark_on(reset_stream);
-            PG2_CUDA(cudaEventRecord(ev_reset_done, reset_stream));   // = main render done
-            PG2_CUDA(cudaStreamWaitEvent(stream, ev_reset_done, 0));
-            launch_render(2, reset_count + 3, stream);
-            launches++;
-            if (prof) prof_mark();
-        } else if (prof || !use_graph) {
-            if (enqueue_main(prof)) return 1;
+        if (!use_graph || prof || overlap_reset) {
+            if (enqueue_step(prof)) return 1;
         } else {
             StepGraph& g = graphs[parity | slot << 1];
-            if (g.exec && g.obs != obs) { cudaGraphExecDestroy(g.exec); cudaGraphDestroy(g.graph); g = StepGraph(); }   // the output buffers moved (pipelined stepping started)
+            if (g.exec && g.outputs != cur) { cudaGraphExecDestroy(g.exec); cudaGraphDestroy(g.graph); g = StepGraph(); }   // pipelined stepping started
             if (!g.exec) {
+                // the capture counts the kernels it records (launch_*): they run in the graph launch below
                 cudaGraph_t graph = nullptr;
-                const int64_t launches0 = launches;
                 PG2_CUDA(cudaStreamBeginCapture(stream, cudaStreamCaptureModeThreadLocal));
-                const int rc = enqueue_main(false);
+                const int rc = enqueue_step(false);
                 const cudaError_t ce = cudaStreamEndCapture(stream, &graph);
-                launches = launches0;
                 if (rc || ce != cudaSuccess || !graph) return fail(std::string("step graph capture failed: ") + cudaGetErrorString(ce));
                 size_t nn = 0;
                 PG2_CUDA(cudaGraphGetNodes(graph, nullptr, &nn));
@@ -616,27 +614,29 @@ struct Engine : EngineBase {
                 for (auto node : nodes) {
                     cudaGraphNodeType ty;
                     cudaKernelNodeParams kp{};
-                    if (cudaGraphNodeGetType(node, &ty) == cudaSuccess && ty == cudaGraphNodeTypeKernel &&
-                        cudaGraphKernelNodeGetParams(node, &kp) == cudaSuccess && kp.func == (void*)k_step<G>) g.step_node = node;
+                    if (cudaGraphNodeGetType(node, &ty) != cudaSuccess || ty != cudaGraphNodeTypeKernel) continue;
+                    g.kernels++;
+                    if (cudaGraphKernelNodeGetParams(node, &kp) == cudaSuccess && kp.func == (void*)k_step<G>) g.step_node = node;
                 }
                 if (!g.step_node) { cudaGraphDestroy(graph); return fail("step graph: k_step node not found"); }
                 PG2_CUDA(cudaGraphInstantiate(&g.exec, graph, 0));
                 g.graph = graph;   // kept: the node handle used to re-point `actions` belongs to it
-                g.actions = actions_dev; g.obs = obs;
-            } else if (g.actions != actions_dev) {
-                cudaKernelNodeParams kp = step_node_params();
-                PG2_CUDA(cudaGraphExecKernelNodeSetParams(g.exec, g.step_node, &kp));
-                g.actions = actions_dev;
+                g.actions = actions_dev; g.outputs = cur;
+            } else {
+                if (g.actions != actions_dev) {
+                    cudaKernelNodeParams kp = step_node_params();
+                    PG2_CUDA(cudaGraphExecKernelNodeSetParams(g.exec, g.step_node, &kp));
+                    g.actions = actions_dev;
+                }
+                launches += g.kernels;
             }
             PG2_CUDA(cudaGraphLaunch(g.exec, stream));
-            launches += prefetch ? 2 : 3;
         }
         if (prefetch) {
             // the level after the one just taken: generated on the slot's own (high-priority) stream from here on
             PG2_CUDA(cudaEventRecord(ev_stepped, stream));
             PG2_CUDA(cudaStreamWaitEvent(prep_streams[slot], ev_stepped, 0));
-            k_reset<G><<<reset_grid(N), 32 * RESET_WARPS_PER_CTA, reset_smem(), prep_streams[slot]>>>(shadow_st, shadow_common, ka_list, ka_count, N, gen_done);
-            launches++;
+            launch_reset(shadow_st, shadow_common, ka_list, ka_count, gen_done, prep_streams[slot]);
             PG2_CUDA(cudaEventRecord(ev_prepared[slot], prep_streams[slot]));
         }
         PG2_CUDA(cudaGetLastError());
@@ -748,27 +748,27 @@ int32_t pg2_step_device(pg2_engine* e, const int32_t* actions_device) {
     return e->impl->step_device(actions_device);
 }
 
-int32_t pg2_fetch(pg2_engine* e, uint8_t* obs, float* reward, uint8_t* terminated, uint8_t* truncated) {
-    EngineBase* b = e->impl.get();
-    PG2_ON_DEVICE(b->device);
-    if (obs) PG2_CUDA(cudaMemcpyAsync(obs, b->obs, (size_t)b->N * OBS_BYTES, cudaMemcpyDeviceToHost, b->stream));
-    if (reward) PG2_CUDA(cudaMemcpyAsync(reward, b->reward, sizeof(float) * b->N, cudaMemcpyDeviceToHost, b->stream));
-    if (terminated) PG2_CUDA(cudaMemcpyAsync(terminated, b->terminated, b->N, cudaMemcpyDeviceToHost, b->stream));
-    if (truncated) PG2_CUDA(cudaMemcpyAsync(truncated, b->truncated, b->N, cudaMemcpyDeviceToHost, b->stream));
-    PG2_CUDA(cudaStreamSynchronize(b->stream));
+// Enqueue the copies of the current results into host buffers (each may be NULL) on `on`.
+static int copy_outputs(const EngineBase* b, uint8_t* obs, float* reward, uint8_t* terminated, uint8_t* truncated, cudaStream_t on) {
+    const EngineBase::Outputs& o = b->out[b->cur];
+    const size_t n = (size_t)b->N;
+    if (obs) PG2_CUDA(cudaMemcpyAsync(obs, o.obs, n * OBS_BYTES, cudaMemcpyDeviceToHost, on));
+    if (reward) PG2_CUDA(cudaMemcpyAsync(reward, o.reward, sizeof(float) * n, cudaMemcpyDeviceToHost, on));
+    if (terminated) PG2_CUDA(cudaMemcpyAsync(terminated, o.terminated, n, cudaMemcpyDeviceToHost, on));
+    if (truncated) PG2_CUDA(cudaMemcpyAsync(truncated, o.truncated, n, cudaMemcpyDeviceToHost, on));
     return 0;
 }
 
 // pg2_fetch without the wait: the copies are enqueued on the engine's stream (truly asynchronous only into page-locked
 // memory, pg2_host_alloc); pg2_sync completes them.
 int32_t pg2_fetch_async(pg2_engine* e, uint8_t* obs, float* reward, uint8_t* terminated, uint8_t* truncated) {
-    EngineBase* b = e->impl.get();
-    PG2_ON_DEVICE(b->device);
-    if (obs) PG2_CUDA(cudaMemcpyAsync(obs, b->obs, (size_t)b->N * OBS_BYTES, cudaMemcpyDeviceToHost, b->stream));
-    if (reward) PG2_CUDA(cudaMemcpyAsync(reward, b->reward, sizeof(float) * b->N, cudaMemcpyDeviceToHost, b->stream));
-    if (terminated) PG2_CUDA(cudaMemcpyAsync(terminated, b->terminated, b->N, cudaMemcpyDeviceToHost, b->stream));
-    if (truncated) PG2_CUDA(cudaMemcpyAsync(truncated, b->truncated, b->N, cudaMemcpyDeviceToHost, b->stream));
-    return 0;
+    PG2_ON_DEVICE(e->impl->device);
+    return copy_outputs(e->impl.get(), obs, reward, terminated, truncated, e->impl->stream);
+}
+
+int32_t pg2_fetch(pg2_engine* e, uint8_t* obs, float* reward, uint8_t* terminated, uint8_t* truncated) {
+    if (pg2_fetch_async(e, obs, reward, terminated, truncated)) return 1;
+    return pg2_sync(e);
 }
 
 // Page-locked host memory for result / action buffers (cudaHostAlloc, portable across devices); NULL on failure.
@@ -785,11 +785,7 @@ void pg2_host_free(void* p) { if (p) cudaFreeHost(p); }
 // double-buffered in HBM so that the copy of step t-1 overlaps the kernels of step t.
 static int enable_pipeline(EngineBase* b) {
     const int N = b->N;
-    b->obs_b[0] = b->obs; b->reward_b[0] = b->reward; b->term_b[0] = b->terminated; b->trunc_b[0] = b->truncated;
-    PG2_CUDA(cudaMalloc(&b->obs_b[1], (size_t)N * OBS_BYTES));
-    PG2_CUDA(cudaMalloc(&b->reward_b[1], sizeof(float) * N));
-    PG2_CUDA(cudaMalloc(&b->term_b[1], N));
-    PG2_CUDA(cudaMalloc(&b->trunc_b[1], N));
+    if (b->alloc_outputs(b->out[1])) return 1;
     PG2_CUDA(cudaStreamCreateWithFlags(&b->copy_stream, cudaStreamNonBlocking));
     for (int k = 0; k < 2; k++) {
         PG2_CUDA(cudaMalloc(&b->actions_b[k], sizeof(int32_t) * N));
@@ -798,7 +794,6 @@ static int enable_pipeline(EngineBase* b) {
         PG2_CUDA(cudaEventCreateWithFlags(&b->ev_copy[k], cudaEventDisableTiming));
         PG2_CUDA(cudaEventCreateWithFlags(&b->ev_h2d[k], cudaEventDisableTiming));
     }
-    b->cur = 0;
     b->pipelined = true;
     return 0;
 }
@@ -814,18 +809,14 @@ int32_t pg2_step_pipelined(pg2_engine* e, const int32_t* actions_host, uint8_t* 
     memcpy(b->pinned_b[slot], actions_host, sizeof(int32_t) * N);
     PG2_CUDA(cudaMemcpyAsync(b->actions_b[slot], b->pinned_b[slot], sizeof(int32_t) * N, cudaMemcpyHostToDevice, b->stream));
     PG2_CUDA(cudaEventRecord(b->ev_h2d[slot], b->stream));
-    b->obs = b->obs_b[slot]; b->reward = b->reward_b[slot]; b->terminated = b->term_b[slot]; b->truncated = b->trunc_b[slot];
+    b->cur = slot;
     if (b->step_device(b->actions_b[slot])) return 1;
     PG2_CUDA(cudaEventRecord(b->ev_step[slot], b->stream));
     PG2_CUDA(cudaStreamWaitEvent(b->copy_stream, b->ev_step[slot], 0));
-    if (obs) PG2_CUDA(cudaMemcpyAsync(obs, b->obs, (size_t)N * OBS_BYTES, cudaMemcpyDeviceToHost, b->copy_stream));
-    if (reward) PG2_CUDA(cudaMemcpyAsync(reward, b->reward, sizeof(float) * N, cudaMemcpyDeviceToHost, b->copy_stream));
-    if (terminated) PG2_CUDA(cudaMemcpyAsync(terminated, b->terminated, N, cudaMemcpyDeviceToHost, b->copy_stream));
-    if (truncated) PG2_CUDA(cudaMemcpyAsync(truncated, b->truncated, N, cudaMemcpyDeviceToHost, b->copy_stream));
+    if (copy_outputs(b, obs, reward, terminated, truncated, b->copy_stream)) return 1;
     PG2_CUDA(cudaEventRecord(b->ev_copy[slot], b->copy_stream));
     b->copy_pending[slot] = true;
     if (b->copy_pending[prev]) PG2_CUDA(cudaEventSynchronize(b->ev_copy[prev]));   // results of the previous call are ready
-    b->cur = slot;
     return 0;
 }
 
@@ -837,10 +828,10 @@ int32_t pg2_pipeline_flush(pg2_engine* e) {
     return 0;
 }
 
-uint8_t* pg2_obs_device(pg2_engine* e) { return e->impl->obs; }
-float* pg2_reward_device(pg2_engine* e) { return e->impl->reward; }
-uint8_t* pg2_terminated_device(pg2_engine* e) { return e->impl->terminated; }
-uint8_t* pg2_truncated_device(pg2_engine* e) { return e->impl->truncated; }
+uint8_t* pg2_obs_device(pg2_engine* e) { return e->impl->out[e->impl->cur].obs; }
+float* pg2_reward_device(pg2_engine* e) { return e->impl->out[e->impl->cur].reward; }
+uint8_t* pg2_terminated_device(pg2_engine* e) { return e->impl->out[e->impl->cur].terminated; }
+uint8_t* pg2_truncated_device(pg2_engine* e) { return e->impl->out[e->impl->cur].truncated; }
 
 int32_t pg2_sync(pg2_engine* e) {
     PG2_ON_DEVICE(e->impl->device);
@@ -914,52 +905,56 @@ int64_t pg2_write_field(pg2_engine* e, const char* name, const void* in, int64_t
     return bytes;
 }
 
-// blob = header { magic, game tag, N, parity, state bytes, common bytes } + state_mem + common_mem + obs + reward +
-// terminated + truncated
+// blob = header { magic, game tag, N, parity, state bytes, common bytes } + the sections of blob_sections, in order
 struct SnapshotHeader { uint32_t magic, game; int32_t n, parity; uint64_t state_bytes, common_bytes; };
 static const uint32_t SNAPSHOT_MAGIC = 0x50473253u;   // "PG2S"
+struct BlobSection { void* dev; size_t bytes; };
+static const int BLOB_SECTIONS = 6;
+
+// The device buffers a blob holds: state_mem, common_mem and the current results. Returns the size of the blob.
+static int64_t blob_sections(EngineBase* b, BlobSection sec[BLOB_SECTIONS]) {
+    const EngineBase::Outputs& o = b->out[b->cur];
+    const size_t n = (size_t)b->N;
+    const BlobSection all[BLOB_SECTIONS] = { { b->state_mem, b->state_alloc_bytes() }, { b->common_mem, CommonState::bytes(b->N) },
+                                             { o.obs, n * OBS_BYTES }, { o.reward, n * sizeof(float) }, { o.terminated, n }, { o.truncated, n } };
+    int64_t total = sizeof(SnapshotHeader);
+    for (int k = 0; k < BLOB_SECTIONS; k++) { sec[k] = all[k]; total += (int64_t)all[k].bytes; }
+    return total;
+}
 
 int64_t pg2_snapshot(pg2_engine* e, void* out, int64_t capacity) {
     EngineBase* b = e->impl.get();
-    const size_t sb = b->state_alloc_bytes(), cb = CommonState::bytes(b->N), n = (size_t)b->N;
-    const int64_t total = (int64_t)(sizeof(SnapshotHeader) + sb + cb + n * OBS_BYTES + n * sizeof(float) + 2 * n);
+    BlobSection sec[BLOB_SECTIONS];
+    const int64_t total = blob_sections(b, sec);
     if (!out) return total;
     if (capacity < total) { g_error = "pg2_snapshot: buffer too small"; return -2; }
     if (b->pipelined) { g_error = "pg2_snapshot: flush the pipelined stepping first (pg2_pipeline_flush) and use pg2_step"; return -2; }
     DeviceGuard guard__(b->device);
     if (cudaStreamSynchronize(b->stream) != cudaSuccess) { g_error = "pg2_snapshot: sync failed"; return -3; }
-    SnapshotHeader h{ SNAPSHOT_MAGIC, b->game_tag(), b->N, b->parity, (uint64_t)sb, (uint64_t)cb };
+    SnapshotHeader h{ SNAPSHOT_MAGIC, b->game_tag(), b->N, b->parity, (uint64_t)sec[0].bytes, (uint64_t)sec[1].bytes };
     char* p = (char*)out;
     memcpy(p, &h, sizeof(h)); p += sizeof(h);
-    bool ok = cudaMemcpy(p, b->state_mem, sb, cudaMemcpyDeviceToHost) == cudaSuccess; p += sb;
-    ok = ok && cudaMemcpy(p, b->common_mem, cb, cudaMemcpyDeviceToHost) == cudaSuccess; p += cb;
-    ok = ok && cudaMemcpy(p, b->obs, n * OBS_BYTES, cudaMemcpyDeviceToHost) == cudaSuccess; p += n * OBS_BYTES;
-    ok = ok && cudaMemcpy(p, b->reward, n * sizeof(float), cudaMemcpyDeviceToHost) == cudaSuccess; p += n * sizeof(float);
-    ok = ok && cudaMemcpy(p, b->terminated, n, cudaMemcpyDeviceToHost) == cudaSuccess; p += n;
-    ok = ok && cudaMemcpy(p, b->truncated, n, cudaMemcpyDeviceToHost) == cudaSuccess;
+    bool ok = true;
+    for (const BlobSection& s : sec) { ok = ok && cudaMemcpy(p, s.dev, s.bytes, cudaMemcpyDeviceToHost) == cudaSuccess; p += s.bytes; }
     if (!ok) { g_error = "pg2_snapshot: copy failed"; return -3; }
     return total;
 }
 
 int64_t pg2_restore(pg2_engine* e, const void* blob, int64_t bytes) {
     EngineBase* b = e->impl.get();
-    const size_t sb = b->state_alloc_bytes(), cb = CommonState::bytes(b->N), n = (size_t)b->N;
-    const int64_t total = (int64_t)(sizeof(SnapshotHeader) + sb + cb + n * OBS_BYTES + n * sizeof(float) + 2 * n);
+    BlobSection sec[BLOB_SECTIONS];
+    const int64_t total = blob_sections(b, sec);
     SnapshotHeader h;
     if (bytes < (int64_t)sizeof(h)) { g_error = "pg2_restore: truncated blob"; return -2; }
     memcpy(&h, blob, sizeof(h));
-    if (h.magic != SNAPSHOT_MAGIC || h.game != b->game_tag() || h.n != b->N || h.state_bytes != sb || h.common_bytes != cb || bytes != total) {
+    if (h.magic != SNAPSHOT_MAGIC || h.game != b->game_tag() || h.n != b->N || h.state_bytes != sec[0].bytes || h.common_bytes != sec[1].bytes || bytes != total) {
         g_error = "pg2_restore: blob does not belong to this game / shard size"; return -2;
     }
     DeviceGuard guard__(b->device);
     if (cudaStreamSynchronize(b->stream) != cudaSuccess) { g_error = "pg2_restore: sync failed"; return -3; }
     const char* p = (const char*)blob + sizeof(h);
-    bool ok = cudaMemcpy(b->state_mem, p, sb, cudaMemcpyHostToDevice) == cudaSuccess; p += sb;
-    ok = ok && cudaMemcpy(b->common_mem, p, cb, cudaMemcpyHostToDevice) == cudaSuccess; p += cb;
-    ok = ok && cudaMemcpy(b->obs, p, n * OBS_BYTES, cudaMemcpyHostToDevice) == cudaSuccess; p += n * OBS_BYTES;
-    ok = ok && cudaMemcpy(b->reward, p, n * sizeof(float), cudaMemcpyHostToDevice) == cudaSuccess; p += n * sizeof(float);
-    ok = ok && cudaMemcpy(b->terminated, p, n, cudaMemcpyHostToDevice) == cudaSuccess; p += n;
-    ok = ok && cudaMemcpy(b->truncated, p, n, cudaMemcpyHostToDevice) == cudaSuccess;
+    bool ok = true;
+    for (const BlobSection& s : sec) { ok = ok && cudaMemcpy(s.dev, p, s.bytes, cudaMemcpyHostToDevice) == cudaSuccess; p += s.bytes; }
     // the reset-list counters are transient within a step: zero them like a fresh engine, keep the parity of the snapshot
     ok = ok && cudaMemset(b->reset_count, 0, 4 * sizeof(int)) == cudaSuccess;
     ok = ok && cudaMemset(b->common.view_valid, 0, (size_t)b->N) == cudaSuccess;   // the view caches are not part of the blob

@@ -22,7 +22,7 @@
 namespace pg2 {
 
 #define PG2_CAVEFLYER_FIELDS_(F, NT)                                                                \
-    F(uint8_t, tiles, NT)       /* env-major [y + x*H]: 0 empty, 1 wall */                         \
+    PG2_ENV_MAJOR(F)(uint8_t, tiles, NT) /* [y + x*H]: 0 empty, 1 wall */                          \
     F(int32_t, num_obj, 1)                                                                         \
     F(uint8_t, obj_type, 64)    /* slot-major; 1 obstacle, 2 target, 3 enemy, 0 destroyed */       \
     F(float, obj_x, 64) F(float, obj_y, 64) F(float, obj_vx, 64) F(float, obj_vy, 64)              \

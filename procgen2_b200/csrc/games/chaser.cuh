@@ -25,8 +25,8 @@ namespace pg2 {
 // CELL: type of a cell index y + x*H (19 x 19 needs 16 bits); NT / NF / NE / NM: capacities of the tile map, the point
 // cells, the sprite entities and the mobs
 #define PG2_CHASER_FIELDS_(F, CELL, NT, NF, NE, NM)                                                \
-    F(uint8_t, tiles, NT)       /* env-major [y + x*H]: 0 empty, 1 wall */                         \
-    F(CELL, free_cells, NF)     /* env-major: System_Tilemap::free_cells after regenerate (the point cells) */ \
+    PG2_ENV_MAJOR(F)(uint8_t, tiles, NT) /* [y + x*H]: 0 empty, 1 wall */                          \
+    PG2_ENV_MAJOR(F)(CELL, free_cells, NF) /* System_Tilemap::free_cells after regenerate (the point cells) */ \
     F(int32_t, num_free, 1)                                                                       \
     F(int32_t, num_ents, 1)     /* sprite entities: orbs, eggs, points */                         \
     F(uint8_t, ent_kind, NE)    /* slot-major: 1 orb, 2 egg/mob, 3 point, 0 destroyed */          \

@@ -18,7 +18,7 @@ namespace pg2 {
 
 // Entity pools are slot-major: field[slot * N + env]. Slot = entity id (creation order).
 #define PG2_CLIMBER_FIELDS(F)                                                                  \
-    F(uint8_t, tiles, 1280)     /* env-major [y + x*64], 20 x 64 */                             \
+    PG2_ENV_MAJOR(F)(uint8_t, tiles, 1280) /* [y + x*64], 20 x 64 */                            \
     F(int32_t, num_ents, 1)                                                                     \
     F(uint8_t, ent_type, 40)    /* 1 mob, 2 point, 0 destroyed */                               \
     F(float, ent_x, 40)                                                                         \

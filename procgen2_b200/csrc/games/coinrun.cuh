@@ -19,7 +19,7 @@ namespace pg2 {
 
 // Entity pools are slot-major: field[slot * N + env] (coalesced across a warp of envs).
 #define PG2_COINRUN_FIELDS(F)                                                                  \
-    F(uint8_t, tiles, 4096)     /* env-major [y + x*64]: Tile_ID | crate_type << 4 */          \
+    PG2_ENV_MAJOR(F)(uint8_t, tiles, 4096) /* [y + x*64]: Tile_ID | crate_type << 4 */         \
     F(int32_t, num_ents, 1)     /* entities created by regenerate (saws, mobs, coin) */         \
     F(uint8_t, ent_type, 40)    /* 1 saw, 2 mob, 3 coin */                                      \
     F(float, ent_x, 40)                                                                         \

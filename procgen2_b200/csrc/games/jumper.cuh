@@ -22,7 +22,7 @@
 namespace pg2 {
 
 #define PG2_JUMPER_FIELDS_(F, NT)                                                                   \
-    F(uint8_t, tiles, NT)       /* env-major [y + x*H]: 0 empty, 1 wall_top, 2 wall_mid */         \
+    PG2_ENV_MAJOR(F)(uint8_t, tiles, NT) /* [y + x*H]: 0 empty, 1 wall_top, 2 wall_mid */          \
     F(int32_t, num_spikes, 1)                                                                      \
     F(uint16_t, spike_cell, 64) /* slot-major */                                                   \
     F(uint8_t, sprite_order, 72) /* iteration order of System_Sprite_Render::entities: 0 goal, k+1 spike k */ \

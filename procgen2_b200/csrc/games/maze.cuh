@@ -16,7 +16,7 @@
 namespace pg2 {
 
 #define PG2_MAZE_FIELDS(F)                                              \
-    F(uint8_t, tiles, 1024)  /* env-major, [y + x*WORLD] (WORLD <= 31), 0 empty 1 wall */ \
+    PG2_ENV_MAJOR(F)(uint8_t, tiles, 1024) /* [y + x*WORLD] (WORLD <= 31), 0 empty 1 wall */ \
     F(float, agent_x, 1)                                                \
     F(float, agent_y, 1)                                                \
     F(uint8_t, face_forward, 1)                                         \

@@ -173,7 +173,7 @@ __device__ __noinline__ void swap_copy(const SwapArgs& a, const CommonState& liv
     for (int i = 0; i < a.table.n; i++) {
         const SwapField f = a.table.f[i];
         if (f.per_env <= nthr && (f.esz == 4 || f.esz == 1)) continue;
-        if (f.esz != 4 && f.esz != 1) {   // odd element sizes (none today)
+        if (f.esz != 4 && f.esz != 1) {   // other element sizes, byte by byte (jumper's uint16_t spike_cell)
             for (int j = tid; j < f.per_env; j += nthr) { const size_t off = elem_off(f, j); for (int bb = 0; bb < f.esz; bb++) f.live[off + bb] = f.shadow[off + bb]; }
             continue;
         }

@@ -1,10 +1,12 @@
-// Structure-of-arrays game state in HBM. Each game lists its fields once with an X-macro
-//     F(type, name, elements_per_env)
-// from which the device-visible struct of array pointers, the allocation size and the carving
-// of one big device allocation are generated. Scalars are indexed [env]; small per-env arrays
-// are either env-major (`name[env * K + i]`, contiguous per env: tile maps, which the renderer
-// reads as a window) or slot-major (`name[i * N + env]`, coalesced across a warp of envs:
-// entity / bullet pools walked by the thread-per-env step kernels) — the game decides.
+// Structure-of-arrays game state in HBM. Each game lists its fields once with an X-macro FIELDS(F) of entries
+//     F(type, name, elements_per_env)                  scalar `name[env]` or slot-major array `name[i * N + env]`
+//                                                      (coalesced across a warp of envs: entity / bullet pools walked
+//                                                      by the thread-per-env step kernels)
+//     PG2_ENV_MAJOR(F)(type, name, elements_per_env)   env-major array `name[env * K + i]` (contiguous per env: tile
+//                                                      maps, which the renderer reads as a window)
+// from which the device-visible struct of array pointers, the allocation size and the carving of one big device
+// allocation are generated. Both kinds of entry expand alike except in for_each_field, which passes the layout on to
+// code that copies one env's elements (the level swap of k_render).
 #pragma once
 #include <stddef.h>
 #include <stdint.h>
@@ -26,7 +28,15 @@ inline size_t align256(size_t x) { return (x + 255) & ~(size_t)255; }
         return true;                                                              \
     }
 
-#define PG2_FIELD_VISIT(type, name, per_env) fn(#name, (void*)this->name, (int)sizeof(type), (int)(per_env));
+#define PG2_FIELD_VISIT(type, name, per_env) fn(#name, (void*)this->name, (int)sizeof(type), (int)(per_env), false);
+
+// An env-major entry names the <generator>_E variant of each generator above.
+#define PG2_ENV_MAJOR(F) F##_E
+#define PG2_FIELD_DECL_E PG2_FIELD_DECL
+#define PG2_FIELD_SIZE_E PG2_FIELD_SIZE
+#define PG2_FIELD_BIND_E PG2_FIELD_BIND
+#define PG2_FIELD_FIND_E PG2_FIELD_FIND
+#define PG2_FIELD_VISIT_E(type, name, per_env) fn(#name, (void*)this->name, (int)sizeof(type), (int)(per_env), true);
 
 #define PG2_DEFINE_STATE(NAME, FIELDS)                                   \
     struct NAME {                                                        \
@@ -58,7 +68,7 @@ inline size_t align256(size_t x) { return (x + 255) & ~(size_t)255; }
 
 // State every game has (Appendix A of SURVEY.md: what survives reset()).
 #define PG2_COMMON_FIELDS(F)                                                                   \
-    F(uint32_t, mt, 624)          /* std::mt19937 state words, env-major */                    \
+    PG2_ENV_MAJOR(F)(uint32_t, mt, 624) /* std::mt19937 state words */                         \
     F(int32_t, mti, 1)            /* position in the state (624 = twist before next draw) */   \
     F(float, cam_x, 1)            /* gr.camera_position (persists across reset, Q10) */        \
     F(float, cam_y, 1)                                                                         \

@@ -12,7 +12,7 @@ constexpr int SC_REPORT = 4;
 
 #define PG2_SYNTH_FIELDS(F)          \
     F(sc_scene, scene, 1)            \
-    F(int32_t, report, SC_REPORT)
+    PG2_ENV_MAJOR(F)(int32_t, report, SC_REPORT)
 
 PG2_DEFINE_STATE(SynthState, PG2_SYNTH_FIELDS)
 
