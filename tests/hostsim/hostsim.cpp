@@ -29,6 +29,10 @@ struct SimBase {
     virtual void step(const int32_t* actions) = 0;
     virtual bool find_field(const char* name, void** ptr, int* esz, int* pe) = 0;
     virtual bool render_human(int env, int width, int height, uint8_t* out) = 0;
+    virtual void invalidate_views() = 0;
+    // every field of the game state, then of CommonState, in declaration order (for_each_field)
+    struct FieldInfo { std::string name; void* ptr; int esz, per_env; bool env_major; };
+    std::vector<FieldInfo> fields;
     int N = 0, max_episode_steps = 0;
     std::vector<uint8_t> obs, terminated, truncated;
     std::vector<float> reward;
@@ -72,6 +76,9 @@ struct Sim : SimBase {
         tex = it->second.first.data();
         atlas = it->second.second.data();
         frame_init_tiletex<G>(*frame, tex);
+        auto add = [&](const char* name, void* p, int esz, int pe, bool em) { fields.push_back(FieldInfo{ name, p, esz, pe, em }); };
+        st.for_each_field(add);
+        c.for_each_field(add);
         for (int e = 0; e < N; e++) seed_body(c, e, base_seed + (uint32_t)e, true);
         for (int e = 0; e < N; e++) reset_body<G>(st, c, e, mt_scratch.data(), arena.data(), 0);
         return true;
@@ -98,6 +105,8 @@ struct Sim : SimBase {
     bool render_human(int env, int width, int height, uint8_t* out) override {
         return render_human_body<G>(st, c, env, *frame, tex, atlas, out, width, height, 0, width * height);
     }
+    // the view cache is this sim's own: state copied in from elsewhere says nothing about it
+    void invalidate_views() override { memset(c.view_valid, 0, (size_t)N); }
 };
 
 static std::string g_err;
@@ -148,5 +157,26 @@ long hs_read_field(void* h, const char* name, void* out, long capacity, int* ele
     memcpy(out, ptr, bytes);
     return bytes;
 }
+// Counterpart of hs_read_field: `bytes` must be the field's whole size. Returns it, -1: unknown field, -2: size mismatch.
+long hs_write_field(void* h, const char* name, const void* in, long bytes) {
+    SimBase* s = (SimBase*)h;
+    void* ptr; int esz, pe;
+    if (!s->find_field(name, &ptr, &esz, &pe)) return -1;
+    if (bytes != (long)esz * pe * s->N) return -2;
+    memcpy(ptr, in, bytes);
+    return bytes;
+}
+int hs_field_count(void* h) { return (int)((SimBase*)h)->fields.size(); }
+// Field i of hs_field_count: its name (copied into name_out, 64 bytes), element size, elements per env and layout
+// (1: env-major `name[env * per_env + k]`, 0: `name[k * N + env]`). Returns 0, or -1 for an index out of range.
+int hs_field_info(void* h, int i, char* name_out, int* esz, int* per_env, int* env_major) {
+    SimBase* s = (SimBase*)h;
+    if (i < 0 || i >= (int)s->fields.size()) return -1;
+    const SimBase::FieldInfo& f = s->fields[i];
+    snprintf(name_out, 64, "%s", f.name.c_str());
+    *esz = f.esz; *per_env = f.per_env; *env_major = f.env_major ? 1 : 0;
+    return 0;
+}
+void hs_invalidate_views(void* h) { ((SimBase*)h)->invalidate_views(); }
 
 }  // extern "C"

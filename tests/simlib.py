@@ -30,6 +30,11 @@ def lib():
             getattr(L, n).argtypes = [ctypes.c_void_p]
         L.hs_read_field.restype = ctypes.c_long
         L.hs_read_field.argtypes = [ctypes.c_void_p, ctypes.c_char_p, ctypes.c_void_p, ctypes.c_long, ctypes.POINTER(ctypes.c_int), ctypes.POINTER(ctypes.c_int)]
+        L.hs_write_field.restype = ctypes.c_long
+        L.hs_write_field.argtypes = [ctypes.c_void_p, ctypes.c_char_p, ctypes.c_void_p, ctypes.c_long]
+        L.hs_field_count.argtypes = [ctypes.c_void_p]
+        L.hs_field_info.argtypes = [ctypes.c_void_p, ctypes.c_int, ctypes.c_char_p] + [ctypes.POINTER(ctypes.c_int)] * 3
+        L.hs_invalidate_views.argtypes = [ctypes.c_void_p]
         L.hs_last_error.restype = ctypes.c_char_p
         _lib = L
     return _lib
@@ -49,6 +54,9 @@ class HostSim:
         rew = np.ctypeslib.as_array(L.hs_reward(self.h), shape=(self.n,)).copy()
         term = np.ctypeslib.as_array(L.hs_terminated(self.h), shape=(self.n,)).copy().astype(bool)
         return obs, rew, term
+
+    def truncated(self):
+        return np.ctypeslib.as_array(lib().hs_truncated(self.h), shape=(self.n,)).copy().astype(bool)
 
     def reset(self, seeds=None):
         if seeds is not None:
@@ -77,7 +85,78 @@ class HostSim:
         L.hs_read_field(self.h, name.encode(), buf.ctypes.data, nbytes, None, None)
         return buf, esz.value, pe.value
 
+    def field_list(self):
+        """[(name, element size, elements per env, env-major)] of every field of the game state and CommonState."""
+        L = lib()
+        out = []
+        name = ctypes.create_string_buffer(64)
+        esz, pe, em = ctypes.c_int(), ctypes.c_int(), ctypes.c_int()
+        for i in range(L.hs_field_count(self.h)):
+            assert L.hs_field_info(self.h, i, name, ctypes.byref(esz), ctypes.byref(pe), ctypes.byref(em)) == 0
+            out.append((name.value.decode(), esz.value, pe.value, bool(em.value)))
+        return out
+
+    def write_field(self, name, data):
+        a = np.ascontiguousarray(data)
+        n = lib().hs_write_field(self.h, name.encode(), a.ctypes.data, a.nbytes)
+        if n == -1:
+            raise KeyError(name)
+        if n != a.nbytes:
+            raise ValueError("hs_write_field %s: %d bytes given" % (name, a.nbytes))
+
+    def invalidate_views(self):
+        """Mark every env's cached view stale (its cache is this sim's own, not that of the state's source)."""
+        lib().hs_invalidate_views(self.h)
+
     def close(self):
         if self.h:
             lib().hs_destroy(self.h)
             self.h = None
+
+
+def transplant(src, sim):
+    """Copy every state field of `src` (a BatchedEnv or a HostSim of the same game, mode, N and max_episode_steps)
+    into the HostSim `sim`, byte for byte: both lay a field out alike at equal N. Checks that `src` knows every field
+    the sim has, with the same element size and count per env. The sim's view caches are invalidated."""
+    for name, esz, pe, _ in sim.field_list():
+        if isinstance(src, HostSim):
+            buf, e2, p2 = src.field(name)
+        else:
+            buf, e2, p2 = src.read_field(name)
+        assert (e2, p2) == (esz, pe), "field %s: %d x %d bytes per env in the source, %d x %d in the host-sim" % (name, p2, e2, pe, esz)
+        sim.write_field(name, buf)
+    sim.invalidate_views()
+
+
+def read_state(src, fields):
+    """{name: raw bytes (uint8 array)} of the given fields (HostSim.field_list() entries) of a BatchedEnv or HostSim."""
+    return {name: (src.field(name) if isinstance(src, HostSim) else src.read_field(name))[0] for name, _, _, _ in fields}
+
+
+def _elem(buf, esz, i):
+    raw = bytes(buf[i * esz:(i + 1) * esz])
+    v = int.from_bytes(raw, "little")
+    if esz == 4:
+        return "%d / %r (0x%08x)" % (np.frombuffer(raw, np.int32)[0], float(np.frombuffer(raw, np.float32)[0]), v)
+    return "%d (0x%0*x)" % (v, 2 * esz, v)
+
+
+def state_diff(want, got, fields, n, skip=(), lane_group=None):
+    """Human-readable report of every field in which `got` differs from `want` (read_state of the same field list at n
+    envs), naming the first differing element of each: env, slot / element index and both values (4-byte elements as
+    int32 and float32, and in hex, which tells -0.0 from 0.0 and NaN payloads apart). `skip`: field names not compared.
+    lane_group(env) -> text added to the env. Empty string: equal."""
+    lines = []
+    for name, esz, pe, env_major in fields:
+        if name in skip:
+            continue
+        a, b = want[name], got[name]
+        if np.array_equal(a, b):
+            continue
+        elem = np.flatnonzero((a.reshape(-1, esz) != b.reshape(-1, esz)).any(axis=1))
+        i = int(elem[0])
+        env, k = (i // pe, i % pe) if env_major else (i % n, i // n)
+        envs = np.unique((elem // pe) if env_major else (elem % n))
+        lines.append("field %s: %d elements of %d envs differ; first env %d%s, element %d: want %s, got %s" % (
+            name, elem.size, envs.size, env, lane_group(env) if lane_group else "", k, _elem(a, esz, i), _elem(b, esz, i)))
+    return "\n".join(lines)
