@@ -21,7 +21,10 @@
  *                 one it does not have makes cenv_make fail),
  *                 "host_copy" (INT, default 1; 0: observations stay device-resident — cenv_step / cenv_reset return
  *                 when the kernels have finished, without the device -> host copy of "screen"; rewards and flags are
- *                 still copied)
+ *                 still copied),
+ *                 "final_observation" (INT, default 0; auto-reset only, cenv_make fails with auto_reset 0: there the
+ *                 "screen" of a finished env already is its terminal frame): also return the frame each finished
+ *                 episode ended in, which auto-reset replaces in "screen" by the first frame of the next episode
  *   actions       key "action", INT, value_buffer_size == num_envs
  *   observations  key "screen", BYTE, num_envs * 12288 values (env-major, 64x64x3 RGB)
  *   step infos    (num_envs > 1 only) "reward" FLOAT[num_envs], "terminated" BYTE[num_envs],
@@ -31,6 +34,11 @@
  *                 address of each device shard's buffer (uint8 [count * 12288] / float [count] / uint8 [count]) and of
  *                 the cudaStream_t its kernels run on; the same addresses come from cenv_device_buffer(key, shard).
  *                 Host result buffers are page-locked.
+ *                 With "final_observation" the step infos add "final_screen_device" (INT[2 * num_devices], as above:
+ *                 uint8 [count * 12288] per shard, also cenv_device_buffer("final_screen", shard)) and, with host_copy,
+ *                 "final_screen" (BYTE[num_envs * 12288]). Row i of either is written in a step iff env i terminated or
+ *                 was truncated in it (the rows of the other envs keep older contents; zero at cenv_make); only those
+ *                 rows are copied to the host.
  * With num_envs == 1 and no extension option the behaviour is the reference's.
  */
 #ifndef PG2_CENV_H
@@ -128,7 +136,8 @@ CENV_API int32_t cenv_render();
 CENV_API void cenv_close();
 
 /* Extension (not in the reference): CUDA device address of the result buffer `key` ("screen" | "reward" | "terminated" |
- * "truncated" | "stream") of device shard `device_index`; NULL if unknown / not made. */
+ * "truncated" | "final_screen" | "stream") of device shard `device_index`; NULL if unknown / not made ("final_screen":
+ * without "final_observation"). */
 CENV_API void* cenv_device_buffer(const char* key, int32_t device_index);
 
 #ifdef __cplusplus

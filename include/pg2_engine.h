@@ -49,6 +49,12 @@ typedef struct {
                                     the reference): -1 = the reference's default, 0 easy, 1 hard, 2 memory / extreme.
                                     Every mode of a game's enum is built (maze / chaser / jumper / caveflyer 0-2, coinrun /
                                     climber / bossfight 0-1); a mode the game does not have makes pg2_create fail */
+    int32_t final_obs;           /* 1: also return the terminal frame of every env that finishes (Gymnasium's final_obs):
+                                    row e of pg2_final_obs_device is written in a step iff env e terminated or was truncated
+                                    in it, with render_game(true) of the state it finished in — what an auto_reset = 0 engine
+                                    returns as that step's observation. Other rows keep older contents (zero at creation);
+                                    pg2_reset does not write any. obs, reward, flags and state are the same as with 0.
+                                    Needs auto_reset = 1 (pg2_create fails otherwise). 0 = off: no buffer, no extra work */
 } pg2_config;
 
 PG2_API int32_t pg2_create(const pg2_config* cfg, pg2_engine** out);
@@ -96,6 +102,14 @@ PG2_API uint8_t* pg2_obs_device(pg2_engine* e);
 PG2_API float* pg2_reward_device(pg2_engine* e);
 PG2_API uint8_t* pg2_terminated_device(pg2_engine* e);
 PG2_API uint8_t* pg2_truncated_device(pg2_engine* e);
+/* final_obs engines: the terminal frames, num_envs * 12288 uint8 like obs (NULL when final_obs is off). */
+PG2_API uint8_t* pg2_final_obs_device(pg2_engine* e);
+
+/* final_obs engines: copy the terminal-frame buffer to host memory and wait (pg2_fetch_final), or enqueue the copies of
+ * the rows with rows[i] != 0 (rows: num_envs host flags, NULL = every row) to the same offsets of `host`, one copy per run
+ * of consecutive rows, completed by pg2_sync (pg2_fetch_final_async). Fail on an engine without final_obs. */
+PG2_API int32_t pg2_fetch_final(pg2_engine* e, uint8_t* host);
+PG2_API int32_t pg2_fetch_final_async(pg2_engine* e, const uint8_t* rows, uint8_t* host);
 
 PG2_API int32_t pg2_sync(pg2_engine* e);
 PG2_API void* pg2_stream(pg2_engine* e);            /* cudaStream_t the engine launches on */
@@ -118,9 +132,9 @@ PG2_API int64_t pg2_read_field(pg2_engine* e, const char* name, void* out, int64
 PG2_API int64_t pg2_write_field(pg2_engine* e, const char* name, const void* in, int64_t bytes);
 
 /* Snapshot / restore of the complete simulation state of the shard (every SoA field incl. the MT19937 streams, the
- * current observations / rewards / done flags): a checkpoint the reference cannot take (SURVEY.md §5, §8f rank 4).
- * pg2_snapshot(e, NULL, 0) returns the blob size; otherwise bytes written, <0 on error. A blob restores only into an
- * engine of the same game and shard size. Stepping after pg2_restore reproduces the steps after pg2_snapshot bit for bit. */
+ * current observations / rewards / done flags, and the terminal frames of a final_obs engine): a checkpoint the reference
+ * cannot take (SURVEY.md §5, §8f rank 4). pg2_snapshot(e, NULL, 0) returns the blob size; otherwise bytes written, <0 on
+ * error. A blob restores only into an engine of the same game, shard size and final_obs setting. Stepping after pg2_restore reproduces the steps after pg2_snapshot bit for bit. */
 PG2_API int64_t pg2_snapshot(pg2_engine* e, void* out, int64_t capacity);
 PG2_API int64_t pg2_restore(pg2_engine* e, const void* blob, int64_t bytes);
 

@@ -59,7 +59,7 @@ def build(force=False, verbose=False, ptxas_info=False):
     deps = _sources()
     if force or _stale(ENGINE, deps):
         cmd = ["nvcc"] + NVCC_FLAGS + os.environ.get("PG2_NVCC_EXTRA", "").split() + (["-Xptxas", "-v"] if ptxas_info else []) + [
-            "-shared", os.path.join(CSRC, "engine.cu"), os.path.join(CSRC, "assets.cpp"),
+            "-shared", os.path.join(CSRC, "engine.cu"), os.path.join(CSRC, "engine_final.cu"), os.path.join(CSRC, "assets.cpp"),
             "-lz", "-ldl", "-o", ENGINE]
         if verbose:
             print(" ".join(cmd))

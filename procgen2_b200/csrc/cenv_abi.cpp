@@ -8,7 +8,7 @@
 //   cenv_step   key "action" INT, step, render, copy observation            (coinrun.cpp:341-391)
 //   cenv_close  frees the library-owned buffers                             (coinrun.cpp:413-441)
 // Extension (documented in include/cenv.h): "num_envs", "device", "num_devices", "max_episode_steps", "auto_reset",
-// "host_copy" make-options; batched "action"/"screen" buffers; per-env results and the DEVICE addresses of the
+// "host_copy", "final_observation" make-options; batched "action"/"screen" buffers; per-env results and the DEVICE addresses of the
 // result buffers as step / reset infos (+ the exported getter cenv_device_buffer). Host result buffers are pinned.
 #include <stdio.h>
 #include <stdlib.h>
@@ -52,33 +52,36 @@ int g_num_envs = 1;
 int g_window_w = 512, g_window_h = 512;   // cenv_render's window (options "width" / "height"; limits: pg2_render_human)
 
 int g_host_copy = 1;              // make-option "host_copy": 0 = observations stay in HBM (read them through the device pointers)
+int g_final = 0;                  // make-option "final_observation": the terminal frames of finished envs as step infos
 
 cenv_key_value g_observation;    // shared by reset_data and step_data, like the reference
 cenv_key_value g_obs_space, g_act_space;
-enum { INFO_REWARD, INFO_TERMINATED, INFO_TRUNCATED, INFO_SCREEN_DEV, INFO_REWARD_DEV, INFO_TERMINATED_DEV, INFO_TRUNCATED_DEV, INFO_STREAM, NUM_INFOS };
-cenv_key_value g_infos[NUM_INFOS];
+enum { INFO_REWARD, INFO_TERMINATED, INFO_TRUNCATED, INFO_SCREEN_DEV, INFO_REWARD_DEV, INFO_TERMINATED_DEV, INFO_TRUNCATED_DEV, INFO_STREAM, NUM_INFOS,
+       INFO_FINAL_SCREEN_DEV = NUM_INFOS, INFO_FINAL_SCREEN };   // the last two: step infos with "final_observation" only
+cenv_key_value g_infos[NUM_INFOS + 2];
 float g_box[2] = { 0.0f, 255.0f };
 int32_t g_nvec[1] = { kNumActions };
 // host result buffers: page-locked (pg2_host_alloc), so the device -> host copies run at full PCIe speed and asynchronously
-uint8_t *g_obs = nullptr, *g_term = nullptr, *g_trunc = nullptr;
+uint8_t *g_obs = nullptr, *g_term = nullptr, *g_trunc = nullptr, *g_final_obs = nullptr;
 float* g_reward = nullptr;
+std::vector<uint8_t> g_done;        // "final_observation": terminated | truncated of the last step, per env
 std::vector<uint8_t> g_frame;
 std::vector<int32_t> g_actions, g_seeds;
-std::vector<int32_t> g_devptr[5];   // per info: (lo, hi) 32-bit halves of one address per device
+std::vector<int32_t> g_devptr[6];   // per info: (lo, hi) 32-bit halves of one address per device (the 6th: final_screen_device)
 
 void free_host() {
-    pg2_host_free(g_obs); pg2_host_free(g_reward); pg2_host_free(g_term); pg2_host_free(g_trunc);
-    g_obs = g_term = g_trunc = nullptr; g_reward = nullptr;
+    pg2_host_free(g_obs); pg2_host_free(g_reward); pg2_host_free(g_term); pg2_host_free(g_trunc); pg2_host_free(g_final_obs);
+    g_obs = g_term = g_trunc = g_final_obs = nullptr; g_reward = nullptr;
 }
 
 // addresses of the device-resident results (they alternate between two buffer sets only in pg2_step_pipelined mode,
 // which this library does not use: constant for the lifetime of the environment)
 void publish_device_pointers() {
-    for (int k = 0; k < 5; k++) g_devptr[k].assign(2 * g_engines.size(), 0);
+    for (int k = 0; k < 6; k++) g_devptr[k].assign(2 * g_engines.size(), 0);
     for (size_t d = 0; d < g_engines.size(); d++) {
-        const void* p[5] = { pg2_obs_device(g_engines[d]), pg2_reward_device(g_engines[d]), pg2_terminated_device(g_engines[d]),
-                             pg2_truncated_device(g_engines[d]), pg2_stream(g_engines[d]) };
-        for (int k = 0; k < 5; k++) {
+        const void* p[6] = { pg2_obs_device(g_engines[d]), pg2_reward_device(g_engines[d]), pg2_terminated_device(g_engines[d]),
+                             pg2_truncated_device(g_engines[d]), pg2_stream(g_engines[d]), pg2_final_obs_device(g_engines[d]) };
+        for (int k = 0; k < 6; k++) {
             const uint64_t a = (uint64_t)(uintptr_t)p[k];
             g_devptr[k][2 * d] = (int32_t)(uint32_t)(a & 0xffffffffu);
             g_devptr[k][2 * d + 1] = (int32_t)(uint32_t)(a >> 32);
@@ -92,6 +95,23 @@ int fetch() {
     for (size_t d = 0; d < g_engines.size(); d++) {
         const size_t o = (size_t)g_first[d];
         if (pg2_fetch_async(g_engines[d], g_host_copy ? g_obs + o * kObsBytes : nullptr, g_reward + o, g_term + o, g_trunc + o)) {
+            fprintf(stderr, "[procgen2_b200] %s\n", pg2_last_error());
+            return 1;
+        }
+    }
+    for (size_t d = 0; d < g_engines.size(); d++)
+        if (pg2_sync(g_engines[d])) { fprintf(stderr, "[procgen2_b200] %s\n", pg2_last_error()); return 1; }
+    return 0;
+}
+
+// "final_observation" with host_copy, after fetch(): the terminal frames of the envs that finished in the step -> the host
+// buffer, one copy per run of consecutive finished envs (the flags are on the host already); the other rows keep their
+// older contents, as on the device.
+int fetch_final() {
+    for (int e = 0; e < g_num_envs; e++) g_done[e] = g_term[e] | g_trunc[e];
+    for (size_t d = 0; d < g_engines.size(); d++) {
+        const size_t o = (size_t)g_first[d];
+        if (pg2_fetch_final_async(g_engines[d], g_done.data() + o, g_final_obs + o * kObsBytes)) {
             fprintf(stderr, "[procgen2_b200] %s\n", pg2_last_error());
             return 1;
         }
@@ -118,7 +138,7 @@ int32_t cenv_make(const char* /*render_mode*/, cenv_option* options, int32_t opt
     destroy_all();
     unsigned int seed = (unsigned int)time(nullptr);     // coinrun.cpp:130
     int device = 0, num_devices = 1, max_episode_steps = 0, auto_reset = -1, distribution_mode = -1;
-    g_num_envs = 1; g_host_copy = 1;
+    g_num_envs = 1; g_host_copy = 1; g_final = 0;
     for (int i = 0; i < options_size; i++) {
         std::string name(options[i].name);
         if (options[i].value_type != CENV_VALUE_TYPE_INT) continue;
@@ -133,6 +153,7 @@ int32_t cenv_make(const char* /*render_mode*/, cenv_option* options, int32_t opt
         else if (name == "auto_reset") auto_reset = v;
         else if (name == "host_copy") g_host_copy = v != 0;
         else if (name == "distribution_mode") distribution_mode = v;
+        else if (name == "final_observation") g_final = v != 0;
     }
     if (g_num_envs < 1 || (long long)g_num_envs * kObsBytes > 2147483647LL) {
         fprintf(stderr, "[procgen2_b200] num_envs out of range for an int32 cenv buffer size\n");
@@ -156,6 +177,7 @@ int32_t cenv_make(const char* /*render_mode*/, cenv_option* options, int32_t opt
         cfg.assets_path = nullptr;
         cfg.auto_reset = auto_reset;
         cfg.distribution_mode = distribution_mode;
+        cfg.final_obs = g_final;
         pg2_engine* e = nullptr;
         if (pg2_create(&cfg, &e)) {
             fprintf(stderr, "[procgen2_b200] cenv_make failed (device %d): %s\n", device + d, pg2_last_error());
@@ -171,7 +193,12 @@ int32_t cenv_make(const char* /*render_mode*/, cenv_option* options, int32_t opt
     g_reward = (float*)pg2_host_alloc(sizeof(float) * (size_t)g_num_envs);
     g_term = (uint8_t*)pg2_host_alloc((size_t)g_num_envs);
     g_trunc = (uint8_t*)pg2_host_alloc((size_t)g_num_envs);
-    if (!g_obs || !g_reward || !g_term || !g_trunc) {
+    if (g_final && g_host_copy) {
+        g_final_obs = (uint8_t*)pg2_host_alloc((size_t)g_num_envs * kObsBytes);
+        if (g_final_obs) memset(g_final_obs, 0, (size_t)g_num_envs * kObsBytes);
+    }
+    g_done.assign(g_num_envs, 0);
+    if (!g_obs || !g_reward || !g_term || !g_trunc || (g_final && g_host_copy && !g_final_obs)) {
         fprintf(stderr, "[procgen2_b200] cenv_make: cannot allocate the pinned host buffers: %s\n", pg2_last_error());
         destroy_all();
         return 1;
@@ -214,10 +241,14 @@ int32_t cenv_make(const char* /*render_mode*/, cenv_option* options, int32_t opt
         g_infos[INFO_SCREEN_DEV + k] = { dev_keys[k], CENV_VALUE_TYPE_INT, (int32_t)g_devptr[k].size(), {} };
         g_infos[INFO_SCREEN_DEV + k].value_buffer.i = g_devptr[k].data();
     }
+    g_infos[INFO_FINAL_SCREEN_DEV] = { "final_screen_device", CENV_VALUE_TYPE_INT, (int32_t)g_devptr[5].size(), {} };
+    g_infos[INFO_FINAL_SCREEN_DEV].value_buffer.i = g_devptr[5].data();
+    g_infos[INFO_FINAL_SCREEN] = { "final_screen", CENV_VALUE_TYPE_BYTE, g_num_envs * kObsBytes, {} };
+    g_infos[INFO_FINAL_SCREEN].value_buffer.b = g_final_obs;
     // the reference's single environment reports no infos (coinrun.cpp:200-202); the batched / device-resident
-    // extension adds the per-env results and the device addresses
-    const bool extended = g_num_envs > 1 || !g_host_copy;
-    step_data.infos_size = extended ? NUM_INFOS : 0;
+    // extension adds the per-env results and the device addresses (+ the terminal frames with "final_observation")
+    const bool extended = g_num_envs > 1 || !g_host_copy || g_final;
+    step_data.infos_size = extended ? NUM_INFOS + (g_final ? (g_host_copy ? 2 : 1) : 0) : 0;
     step_data.infos = extended ? g_infos : nullptr;
     reset_data.infos_size = extended ? 5 : 0;
     reset_data.infos = extended ? g_infos + INFO_SCREEN_DEV : nullptr;
@@ -270,6 +301,7 @@ int32_t cenv_step(cenv_key_value* actions, int32_t actions_size) {
             return 1;
         }
     if (fetch()) return 1;
+    if (g_final && g_host_copy && fetch_final()) return 1;
     step_data.reward.f = g_reward[0];
     step_data.terminated = g_term[0] != 0;
     step_data.truncated = g_trunc[0] != 0;
@@ -293,8 +325,8 @@ void cenv_close() {
 }
 
 // Device address of a result buffer of device shard `device_index` (0 .. num_devices - 1): key = "screen" (uint8
-// [count * 12288]), "reward" (float [count]), "terminated" / "truncated" (uint8 [count]) or "stream" (the cudaStream_t the
-// shard's kernels run on). The same addresses are published as the INT-pair infos "<key>_device". NULL if unknown.
+// [count * 12288]), "reward" (float [count]), "terminated" / "truncated" (uint8 [count]), "final_screen" (uint8
+// [count * 12288], with "final_observation") or "stream" (the cudaStream_t the shard's kernels run on). The same addresses are published as the INT-pair infos "<key>_device". NULL if unknown.
 void* cenv_device_buffer(const char* key, int32_t device_index) {
     if (!g_engine || !key || device_index < 0 || (size_t)device_index >= g_engines.size()) return nullptr;
     pg2_engine* e = g_engines[device_index];
@@ -304,6 +336,7 @@ void* cenv_device_buffer(const char* key, int32_t device_index) {
     if (k == "terminated") return pg2_terminated_device(e);
     if (k == "truncated") return pg2_truncated_device(e);
     if (k == "stream") return pg2_stream(e);
+    if (k == "final_screen") return pg2_final_obs_device(e);   // NULL without "final_observation"
     return nullptr;
 }
 

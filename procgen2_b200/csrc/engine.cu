@@ -7,6 +7,7 @@
 //   k_reset<G>   warp-per-finished-env: reset() with on-device procedural level generation,
 //                continuing the env's MT19937 stream                <- reset()     (<g>.cpp)
 //   k_render<G>  CTA-per-env: 64x64x3 observation, TMA bulk store    <- render_game (<g>.cpp) + SDL
+// (final_obs engines draw the terminal frames of finished envs too: k_render_final<G>, engine_final.cu, see enqueue_step)
 // No CPU fallback exists: every entry point fails loudly when CUDA is unavailable.
 #include <cuda_runtime.h>
 #include <stdio.h>
@@ -152,6 +153,15 @@ __global__ void __launch_bounds__(32 * RESET_WARPS_PER_CTA) k_reset(typename G::
     }
 }
 
+// k_render_final<G> (engine_final.cu)
+cudaError_t final_set_sort_table(const uint8_t* table);
+template <class G>
+cudaError_t render_final_occupancy(int* ctas_per_sm);
+template <class G>
+void launch_render_final(int grid, cudaStream_t on, const typename G::State& s, const CommonState& c, const TexInfo* tex, const uint32_t* atlas,
+                         uint8_t* obs, int* ticket, int mode, const int* list, const int* list_count, const uint8_t* pending, int N,
+                         uint8_t* view_cache, const SwapArgs& swap, uint8_t* final_obs, int* zero_ticket);
+
 // ------------------------------------------------------------------------------------------------
 // host engine
 
@@ -170,6 +180,7 @@ static int ensure_sort_table(int device) {
     PG2_CUDA(cudaMemcpy(dev_table, table.data(), table.size(), cudaMemcpyHostToDevice));
     const uint8_t* p = dev_table;
     PG2_CUDA(cudaMemcpyToSymbol(g_sort_perm, &p, sizeof(p)));
+    PG2_CUDA(final_set_sort_table(p));   // the same symbol of engine_final.cu's device code
     PG2_CUDA(cudaDeviceSynchronize());
     done[device] = true;
     return 0;
@@ -188,25 +199,30 @@ struct EngineBase {
     virtual int destroy_graphs() = 0;           // the captured step graphs (they hold pointers into this engine's buffers)
 
     int device = 0, N = 0, max_episode_steps = 0, auto_reset = 1;
+    bool final_on = false;     // pg2_config::final_obs: finished envs' terminal frames go to out[cur].final_obs
     uint32_t base_seed = 0;
     cudaStream_t stream = nullptr;
     int64_t launches = 0;
     int num_sms = 148;
     int step_epw = 1;          // environments per warp in k_step
     int render_ctas_per_sm = 8;   // resident CTAs of k_render per SM (occupancy query)
+    int final_ctas_per_sm = 8;    // ... of k_render_final (final_on)
     // device buffers
     void* state_mem = nullptr;
     void* common_mem = nullptr;
     CommonState common;
     // The results of a step. Set 0 is allocated by init and is the only one until pipelined stepping starts; then the
     // steps alternate between the two sets. out[cur] is the set the last step wrote (and the device pointers expose).
-    struct Outputs { uint8_t* obs = nullptr; float* reward = nullptr; uint8_t* terminated = nullptr; uint8_t* truncated = nullptr; };
+    // final_obs (final_on only): row e = the terminal frame of env e, written in the steps in which env e finished.
+    struct Outputs { uint8_t* obs = nullptr; float* reward = nullptr; uint8_t* terminated = nullptr; uint8_t* truncated = nullptr;
+                     uint8_t* final_obs = nullptr; };
     Outputs out[2];
     int cur = 0;
     int32_t* actions = nullptr;
     int32_t* seeds_dev = nullptr;
     int* reset_list = nullptr;
     int* reset_count = nullptr;      // device counters int[4], see k_step
+    int* final_ticket = nullptr;     // final_on without level prefetch: int[2], the terminal-frame pass's ticket by step parity
     uint8_t* pending = nullptr;      // env is in this step's reset list
     int parity = 0;
     bool overlap_reset = false;      // k_reset on a second stream, concurrent with the render of the other envs
@@ -283,6 +299,10 @@ struct EngineBase {
         PG2_CUDA(cudaMalloc(&o.reward, sizeof(float) * N));
         PG2_CUDA(cudaMalloc(&o.terminated, N));
         PG2_CUDA(cudaMalloc(&o.truncated, N));
+        if (final_on) {
+            PG2_CUDA(cudaMalloc(&o.final_obs, (size_t)N * OBS_BYTES));
+            PG2_CUDA(cudaMemsetAsync(o.final_obs, 0, (size_t)N * OBS_BYTES, stream));   // rows are written only when an env finishes
+        }
         return 0;
     }
 
@@ -290,7 +310,8 @@ struct EngineBase {
         DeviceGuard guard(device);
         if (stream) cudaStreamSynchronize(stream);
         if (pipelined) cudaStreamSynchronize(copy_stream);
-        for (Outputs& o : out) { cudaFree(o.obs); cudaFree(o.reward); cudaFree(o.terminated); cudaFree(o.truncated); }
+        for (Outputs& o : out) { cudaFree(o.obs); cudaFree(o.reward); cudaFree(o.terminated); cudaFree(o.truncated); cudaFree(o.final_obs); }
+        cudaFree(final_ticket);
         cudaFree(state_mem); cudaFree(common_mem); cudaFree(actions); cudaFree(seeds_dev); cudaFree(reset_list); cudaFree(reset_count); cudaFree(view_cache);
         for (int j = 0; j < PREP_SLOTS; j++) if (prep_streams[j]) { cudaStreamSynchronize(prep_streams[j]); cudaStreamDestroy(prep_streams[j]); }
         for (int j = 0; j < PREP_SLOTS; j++) if (ev_prepared[j]) cudaEventDestroy(ev_prepared[j]);
@@ -316,6 +337,7 @@ struct Engine : EngineBase {
 
     int init(const pg2_config* cfg) {
         device = cfg->device; N = cfg->num_envs; max_episode_steps = cfg->max_episode_steps; auto_reset = cfg->auto_reset;
+        final_on = cfg->final_obs != 0;
         base_seed = (uint32_t)cfg->seed + (uint32_t)cfg->first_env;
         PG2_CUDA(cudaSetDevice(device));
         cudaDeviceProp prop;
@@ -350,6 +372,10 @@ struct Engine : EngineBase {
         PG2_CUDA(cudaMemsetAsync(reset_count, 0, 4 * sizeof(int), stream));
         PG2_CUDA(cudaMalloc(&pending, N));
         PG2_CUDA(cudaMemsetAsync(pending, 0, N, stream));
+        if (final_on) {
+            PG2_CUDA(cudaMalloc(&final_ticket, 2 * sizeof(int)));
+            PG2_CUDA(cudaMemsetAsync(final_ticket, 0, 2 * sizeof(int), stream));
+        }
         prefetch = G::PREFETCH_LEVELS && auto_reset && !(max_episode_steps > 0 && max_episode_steps < G::PREFETCH_MIN_EPISODE);
         if (const char* o = getenv("PG2_PREFETCH")) prefetch = atoi(o) != 0 && G::PREFETCH_LEVELS && auto_reset;
         if (prefetch) {
@@ -400,6 +426,11 @@ struct Engine : EngineBase {
         PG2_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&render_ctas_per_sm, k_render<G>, RENDER_THREADS, 0));
         if (render_ctas_per_sm < 1) render_ctas_per_sm = 1;
         if (const char* o = getenv("PG2_RENDER_CTAS_PER_SM")) render_ctas_per_sm = atoi(o) > 0 ? atoi(o) : render_ctas_per_sm;
+        if (final_on) {
+            PG2_CUDA(render_final_occupancy<G>(&final_ctas_per_sm));
+            if (final_ctas_per_sm < 1) final_ctas_per_sm = 1;
+            if (const char* o = getenv("PG2_RENDER_CTAS_PER_SM")) final_ctas_per_sm = atoi(o) > 0 ? atoi(o) : final_ctas_per_sm;
+        }
         // cenv_make: seed, then reset() once (level #1 is generated and never rendered, Q29)
         k_seed<<<(N + 127) / 128, 128, 0, stream>>>(common, N, base_seed, nullptr, 1);
         launches++;
@@ -479,13 +510,22 @@ struct Engine : EngineBase {
         k_reset<G><<<reset_grid(N), 32 * RESET_WARPS_PER_CTA, reset_smem(), on>>>(s, c, list, count, N, gen_done);
         launches++;
     }
-    void launch_render(int mode, int* ticket, cudaStream_t on) {
-        const int per_sm = render_ctas_per_sm;
+    // final: a step of a final_on engine. With level prefetch the render of the step draws the terminal frames too (mode 0);
+    // without it, final is the pass over the reset list before k_reset (mode 2) that writes the terminal frames.
+    void launch_render(int mode, int* ticket, cudaStream_t on, bool final = false) {
+        const int per_sm = final ? final_ctas_per_sm : render_ctas_per_sm;
         int grid = N < num_sms * per_sm ? N : num_sms * per_sm;
         // (level prefetch: the list / counter k_step appended this step's finished envs to)
         const int* lst = prefetch && ka_list ? ka_list : reset_list;
         const int* cnt = prefetch && ka_count ? ka_count : reset_count + parity;
-        k_render<G><<<grid, RENDER_THREADS, 0, on>>>(st, common, texinfo, atlas, out[cur].obs, ticket, mode, lst, cnt, pending, N, view_cache, swap_args);
+        if (!final)
+            k_render<G><<<grid, RENDER_THREADS, 0, on>>>(st, common, texinfo, atlas, out[cur].obs, ticket, mode, lst, cnt, pending, N, view_cache, swap_args);
+        else if (prefetch)
+            launch_render_final<G>(grid, on, st, common, texinfo, atlas, out[cur].obs, ticket, mode, lst, cnt, pending, N, view_cache, swap_args,
+                                   out[cur].final_obs, nullptr);
+        else
+            launch_render_final<G>(grid, on, st, common, texinfo, atlas, out[cur].final_obs, ticket, mode, lst, cnt, pending, N, view_cache, swap_args,
+                                   nullptr, final_ticket + (parity ^ 1));
         launches++;
     }
 
@@ -523,6 +563,13 @@ struct Engine : EngineBase {
     // WHILE a second stream renders all other envs, a short tail render of the reset envs follows (eager only).
     // Timing marks (pg2_profile, eager): [0] k_step, [1] k_reset on the main stream, [2] render (overlap_reset: the
     // render on the second stream; the wait for it and the tail render are not counted).
+    // final_on: the terminal frame of a finished env is drawn from the state it finished in, before any reset touches it.
+    // With level prefetch that state is still live when the render starts, and the render CTA that swaps the env's level
+    // in draws the terminal frame first (k_render_final, no extra launch). Otherwise k_reset overwrites it, so a pass of
+    // k_render_final over the reset list runs between k_step and k_reset (one more launch; its time counts as [1]). On the
+    // overlap_reset schedule the pass runs before the fork: after it, between the fork and k_reset, it would delay k_reset
+    // until the render of the other envs, which fills the SMs meanwhile, has finished (chaser 4096: +55 % per step).
+    // The pass's ticket alternates with the step parity: each pass zeroes the one the next step uses.
     SwapArgs swap_args;             // table.n == 0 when the engine does not prefetch levels
     const int32_t* ka_actions = nullptr;
     int *ka_list = nullptr, *ka_count = nullptr, *ka_zero_a = nullptr, *ka_zero_b = nullptr;
@@ -557,6 +604,7 @@ struct Engine : EngineBase {
         if (prof) prof_mark();
         if (launch_step(stream)) return 1;
         if (prof) prof_mark();
+        if (final_on && !prefetch) launch_render(2, final_ticket + parity, stream, true);
         if (overlap_reset) {   // fork: the render of all OTHER envs runs on the second stream
             PG2_CUDA(cudaEventRecord(ev_stepped, stream));
             PG2_CUDA(cudaStreamWaitEvent(reset_stream, ev_stepped, 0));
@@ -573,7 +621,7 @@ struct Engine : EngineBase {
             PG2_CUDA(cudaStreamWaitEvent(stream, ev_reset_done, 0));
             launch_render(2, reset_count + 3, stream);
         } else {
-            launch_render(0, reset_count + 2, stream);
+            launch_render(0, reset_count + 2, stream, final_on && prefetch);
         }
         if (prof) prof_mark();
         return 0;
@@ -692,6 +740,8 @@ const char* pg2_last_error(void) { return g_error.c_str(); }
 int32_t pg2_create(const pg2_config* cfg, pg2_engine** out) {
     if (!cfg || !out || !cfg->game) return fail("pg2_create: null argument");
     if (cfg->num_envs <= 0) return fail("pg2_create: num_envs must be positive");
+    if (cfg->final_obs && !cfg->auto_reset)
+        return fail("pg2_create: final_obs needs auto_reset = 1 (with auto_reset = 0 the step's observation already is the terminal frame)");
     int ndev = 0;
     if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
         return fail("pg2_create: no CUDA device available — this engine has no CPU fallback");
@@ -832,6 +882,29 @@ uint8_t* pg2_obs_device(pg2_engine* e) { return e->impl->out[e->impl->cur].obs; 
 float* pg2_reward_device(pg2_engine* e) { return e->impl->out[e->impl->cur].reward; }
 uint8_t* pg2_terminated_device(pg2_engine* e) { return e->impl->out[e->impl->cur].terminated; }
 uint8_t* pg2_truncated_device(pg2_engine* e) { return e->impl->out[e->impl->cur].truncated; }
+uint8_t* pg2_final_obs_device(pg2_engine* e) { return e->impl->out[e->impl->cur].final_obs; }
+
+int32_t pg2_fetch_final_async(pg2_engine* e, const uint8_t* rows, uint8_t* host) {
+    const EngineBase* b = e->impl.get();
+    if (!b->final_on) return fail("pg2_fetch_final: the engine was created without final_obs");
+    if (!host) return fail("pg2_fetch_final: null argument");
+    PG2_ON_DEVICE(b->device);
+    const uint8_t* src = b->out[b->cur].final_obs;
+    for (int i = 0; i < b->N;) {
+        if (rows && !rows[i]) { i++; continue; }
+        int j = i + 1;
+        while (j < b->N && (!rows || rows[j])) j++;
+        const size_t off = (size_t)i * OBS_BYTES;
+        PG2_CUDA(cudaMemcpyAsync(host + off, src + off, (size_t)(j - i) * OBS_BYTES, cudaMemcpyDeviceToHost, b->stream));
+        i = j;
+    }
+    return 0;
+}
+
+int32_t pg2_fetch_final(pg2_engine* e, uint8_t* host) {
+    if (pg2_fetch_final_async(e, nullptr, host)) return 1;
+    return pg2_sync(e);
+}
 
 int32_t pg2_sync(pg2_engine* e) {
     PG2_ON_DEVICE(e->impl->device);
@@ -909,23 +982,28 @@ int64_t pg2_write_field(pg2_engine* e, const char* name, const void* in, int64_t
 struct SnapshotHeader { uint32_t magic, game; int32_t n, parity; uint64_t state_bytes, common_bytes; };
 static const uint32_t SNAPSHOT_MAGIC = 0x50473253u;   // "PG2S"
 struct BlobSection { void* dev; size_t bytes; };
-static const int BLOB_SECTIONS = 6;
+static const int BLOB_SECTIONS = 7;
 
-// The device buffers a blob holds: state_mem, common_mem and the current results. Returns the size of the blob.
-static int64_t blob_sections(EngineBase* b, BlobSection sec[BLOB_SECTIONS]) {
+// The device buffers a blob holds: state_mem, common_mem and the current results (final_obs only when the engine has it:
+// a blob restores only into an engine with the same setting, which the size check enforces). Returns the size of the
+// blob; *nsec = the number of sections.
+static int64_t blob_sections(EngineBase* b, BlobSection sec[BLOB_SECTIONS], int* nsec) {
     const EngineBase::Outputs& o = b->out[b->cur];
     const size_t n = (size_t)b->N;
     const BlobSection all[BLOB_SECTIONS] = { { b->state_mem, b->state_alloc_bytes() }, { b->common_mem, CommonState::bytes(b->N) },
-                                             { o.obs, n * OBS_BYTES }, { o.reward, n * sizeof(float) }, { o.terminated, n }, { o.truncated, n } };
+                                             { o.obs, n * OBS_BYTES }, { o.reward, n * sizeof(float) }, { o.terminated, n }, { o.truncated, n },
+                                             { o.final_obs, n * OBS_BYTES } };
+    *nsec = b->final_on ? 7 : 6;
     int64_t total = sizeof(SnapshotHeader);
-    for (int k = 0; k < BLOB_SECTIONS; k++) { sec[k] = all[k]; total += (int64_t)all[k].bytes; }
+    for (int k = 0; k < *nsec; k++) { sec[k] = all[k]; total += (int64_t)all[k].bytes; }
     return total;
 }
 
 int64_t pg2_snapshot(pg2_engine* e, void* out, int64_t capacity) {
     EngineBase* b = e->impl.get();
     BlobSection sec[BLOB_SECTIONS];
-    const int64_t total = blob_sections(b, sec);
+    int nsec = 0;
+    const int64_t total = blob_sections(b, sec, &nsec);
     if (!out) return total;
     if (capacity < total) { g_error = "pg2_snapshot: buffer too small"; return -2; }
     if (b->pipelined) { g_error = "pg2_snapshot: flush the pipelined stepping first (pg2_pipeline_flush) and use pg2_step"; return -2; }
@@ -935,7 +1013,7 @@ int64_t pg2_snapshot(pg2_engine* e, void* out, int64_t capacity) {
     char* p = (char*)out;
     memcpy(p, &h, sizeof(h)); p += sizeof(h);
     bool ok = true;
-    for (const BlobSection& s : sec) { ok = ok && cudaMemcpy(p, s.dev, s.bytes, cudaMemcpyDeviceToHost) == cudaSuccess; p += s.bytes; }
+    for (int k = 0; k < nsec; k++) { ok = ok && cudaMemcpy(p, sec[k].dev, sec[k].bytes, cudaMemcpyDeviceToHost) == cudaSuccess; p += sec[k].bytes; }
     if (!ok) { g_error = "pg2_snapshot: copy failed"; return -3; }
     return total;
 }
@@ -943,7 +1021,8 @@ int64_t pg2_snapshot(pg2_engine* e, void* out, int64_t capacity) {
 int64_t pg2_restore(pg2_engine* e, const void* blob, int64_t bytes) {
     EngineBase* b = e->impl.get();
     BlobSection sec[BLOB_SECTIONS];
-    const int64_t total = blob_sections(b, sec);
+    int nsec = 0;
+    const int64_t total = blob_sections(b, sec, &nsec);
     SnapshotHeader h;
     if (bytes < (int64_t)sizeof(h)) { g_error = "pg2_restore: truncated blob"; return -2; }
     memcpy(&h, blob, sizeof(h));
@@ -954,9 +1033,10 @@ int64_t pg2_restore(pg2_engine* e, const void* blob, int64_t bytes) {
     if (cudaStreamSynchronize(b->stream) != cudaSuccess) { g_error = "pg2_restore: sync failed"; return -3; }
     const char* p = (const char*)blob + sizeof(h);
     bool ok = true;
-    for (const BlobSection& s : sec) { ok = ok && cudaMemcpy(s.dev, p, s.bytes, cudaMemcpyHostToDevice) == cudaSuccess; p += s.bytes; }
+    for (int k = 0; k < nsec; k++) { ok = ok && cudaMemcpy(sec[k].dev, p, sec[k].bytes, cudaMemcpyHostToDevice) == cudaSuccess; p += sec[k].bytes; }
     // the reset-list counters are transient within a step: zero them like a fresh engine, keep the parity of the snapshot
     ok = ok && cudaMemset(b->reset_count, 0, 4 * sizeof(int)) == cudaSuccess;
+    if (b->final_ticket) ok = ok && cudaMemset(b->final_ticket, 0, 2 * sizeof(int)) == cudaSuccess;
     ok = ok && cudaMemset(b->common.view_valid, 0, (size_t)b->N) == cudaSuccess;   // the view caches are not part of the blob
     b->parity = h.parity;
     if (!ok) { g_error = "pg2_restore: copy failed"; return -3; }

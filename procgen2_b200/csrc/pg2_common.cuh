@@ -128,13 +128,13 @@ PG2_DEV Axis make_axis_inl(float pos, float cam, float cs, float size, int tex_l
     return a;
 }
 
-PG2_DEV_CALL Axis make_axis(float pos, float cam, float cs, float size, int tex_len, float scale, bool flip, bool y_axis) {
+PG2_TU_LOCAL PG2_DEV_CALL Axis make_axis(float pos, float cam, float cs, float size, int tex_len, float scale, bool flip, bool y_axis) {
     return make_axis_inl(pos, cam, cs, size, tex_len, scale, flip, y_axis);
 }
 
 // Both axes of Renderer::render_texture in one function body: the two chains are independent, so their long
 // dependent float sequences interleave (twice the instruction-level parallelism of two make_axis calls).
-PG2_DEV_CALL void make_axis_xy(float px, float py, float cam_x, float cam_y, float cs, float size_x, float size_y, int tex_w, int tex_h,
+PG2_TU_LOCAL PG2_DEV_CALL void make_axis_xy(float px, float py, float cam_x, float cam_y, float cs, float size_x, float size_y, int tex_w, int tex_h,
                                    float scale, bool flip_h, Axis* ax, Axis* ay) {
     *ax = make_axis_inl(px, cam_x, cs, size_x, tex_w, scale, flip_h, false);
     *ay = make_axis_inl(py, cam_y, cs, size_y, tex_h, scale, false, true);

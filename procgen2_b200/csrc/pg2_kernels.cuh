@@ -9,7 +9,7 @@
 namespace pg2 {
 
 // rng.seed(seed) + process-lifetime defaults (cenv_make)
-PG2_DEV_NOINLINE void seed_body(const CommonState& c, int env, uint32_t seed, bool init_persistent) {
+PG2_TU_LOCAL PG2_DEV_NOINLINE void seed_body(const CommonState& c, int env, uint32_t seed, bool init_persistent) {
     mt_seed(c.mt + (size_t)env * MT_N, seed);
     c.mti[env] = MT_N;
     if (init_persistent) {
@@ -146,7 +146,7 @@ struct SwapArgs {
 // in batches before their stores (the compiler cannot prove that a store does not alias the next load, which would
 // serialise one memory round trip per element): short fields (<= blockDim elements per env) eight fields per round, one
 // element per thread; long ones (tile map, MT19937 words, particle pools) eight elements per thread per round.
-__device__ __noinline__ void swap_copy(const SwapArgs& a, const CommonState& live_c, int env, int N) {
+PG2_TU_LOCAL __device__ __noinline__ void swap_copy(const SwapArgs& a, const CommonState& live_c, int env, int N) {
     const int tid = threadIdx.x, nthr = CTA_THREADS;   // called by the render CTA
     __threadfence();
     auto elem_off = [&](const SwapField& f, int j) { return f.env_major ? ((size_t)env * f.per_env + j) * f.esz : ((size_t)j * N + env) * f.esz; };
@@ -258,6 +258,70 @@ __global__ void __launch_bounds__(RENDER_THREADS, G::RENDER_MIN_CTAS) k_render(t
         if (threadIdx.x == 0) take_ticket();
         if (do_swap) swap_copy(swap, c, env, N);
         render_body<G>(s, c, env, f, tex, atlas, obs, view_cache, false);
+    }
+    if ((threadIdx.x & 31) == 0) frame_store_wait();   // every warp issued bulk stores of its own
+}
+
+// k_render of an engine created with final_obs (Engine::final_on), which returns the terminal frame of every env that
+// finishes. Two uses:
+//   - level prefetch, mode 0 with the swap list: the CTA of a finished env draws two frames, first the terminal frame from
+//     the state the episode ended in into final_obs (a static-view game may load its cached base image: it is still the
+//     episode's own), then, after the level swap, the reset frame into obs;
+//   - inline reset, mode 2 over the reset list between k_step and k_reset: obs = the terminal frames, no swap.
+// Block 0 zeroes *zero_ticket when given: the ticket of the next such launch. The loop is k_render's with those two
+// additions; it is a kernel of its own, compiled in its own translation unit (engine_final.cu), so that the kernels of
+// every engine without final_obs stay exactly what they are.
+template <class G>
+__global__ void __launch_bounds__(RENDER_THREADS, G::RENDER_MIN_CTAS) k_render_final(typename G::State s, CommonState c, const TexInfo* __restrict__ tex,
+                                                           const uint32_t* __restrict__ atlas, uint8_t* __restrict__ obs,
+                                                           int* __restrict__ ticket, int mode, const int* __restrict__ list,
+                                                           const int* __restrict__ list_count, const uint8_t* __restrict__ pending, int N,
+                                                           uint8_t* __restrict__ view_cache, const __grid_constant__ SwapArgs swap,
+                                                           uint8_t* __restrict__ final_obs, int* __restrict__ zero_ticket) {
+    __shared__ FrameOf<G> f;
+    __shared__ int s_env, s_swap;
+    if (zero_ticket != nullptr && blockIdx.x == 0 && threadIdx.x == 0) *zero_ticket = 0;
+    const int count = mode == 2 ? *list_count : N;
+    frame_init_tiletex<G>(f, tex);
+    int next_env = -1;
+    bool next_reuse = false, next_swap = false;
+    const int nfirst = (swap.table.n > 0 && mode == 0) ? *list_count : 0;
+    auto take_ticket = [&]() {
+        int t = atomicAdd(ticket, 1);
+        if (nfirst > 0) {
+            if (t < nfirst) {   // a finished env: its first frame is the terminal frame
+                next_env = list[t]; next_swap = true;
+                next_reuse = G::STATIC_VIEW && view_cache != nullptr && c.view_valid[next_env] != 0;
+                return;
+            }
+            t -= nfirst;
+            while (t < count && pending[t]) t = atomicAdd(ticket, 1) - nfirst;
+        }
+        next_env = t < count ? (mode == 2 ? list[t] : t) : -1;
+        next_swap = false;
+        next_reuse = G::STATIC_VIEW && view_cache != nullptr && next_env >= 0 && c.view_valid[next_env] != 0;
+    };
+    if (threadIdx.x == 0) take_ticket();
+    for (;;) {
+        __syncthreads();   // every warp is done with the previous frame (bands are stored per warp, without a CTA barrier)
+        if (threadIdx.x == 0) { s_env = next_env; s_swap = next_swap ? 1 : 0; }
+        frame_begin(f, next_reuse);
+        __syncthreads();
+        const int env = s_env;
+        if (env < 0) break;
+        const bool do_swap = s_swap != 0;
+        if (threadIdx.x == 0) take_ticket();
+        // one render_body call site for both frames of a finished env: a second inlined copy spills registers
+        uint8_t* dst = do_swap ? final_obs : obs;
+        for (;;) {
+            render_body<G>(s, c, env, f, tex, atlas, dst, view_cache, false);
+            if (dst == obs) break;
+            __syncthreads();   // the same barriers as between two frames of the loop
+            frame_begin(f, false);
+            __syncthreads();
+            swap_copy(swap, c, env, N);
+            dst = obs;
+        }
     }
     if ((threadIdx.x & 31) == 0) frame_store_wait();   // every warp issued bulk stores of its own
 }

@@ -57,7 +57,7 @@ PG2_DEV void sincosf_poly(double xs, double x2, int table, int n, float* sinp, f
     else       { *sinp = sv; *cosp = cv; }
 }
 
-PG2_DEV_CALL void glibc_sincosf(float y, float* sinp, float* cosp) {
+PG2_TU_LOCAL PG2_DEV_CALL void glibc_sincosf(float y, float* sinp, float* cosp) {
     uint32_t xi = __float_as_uint(y);
     uint32_t top = (xi >> 20) & 0x7ffu;                 // abstop12
     double x = (double)y;
@@ -140,7 +140,7 @@ PG2_DEV float glibc_atanf(float x) {
     return hx < 0 ? -z : z;
 }
 
-PG2_DEV_CALL float glibc_atan2f(float y, float x) {
+PG2_TU_LOCAL PG2_DEV_CALL float glibc_atan2f(float y, float x) {
     const float tiny = 1.0e-30f, pi_o_4 = 7.8539818525e-01f, pi_o_2 = 1.5707963705e+00f, pi = 3.1415927410e+00f, pi_lo = -8.7422776573e-08f;
     int32_t hx = (int32_t)__float_as_uint(x), hy = (int32_t)__float_as_uint(y);
     int32_t ix = hx & 0x7fffffff, iy = hy & 0x7fffffff;

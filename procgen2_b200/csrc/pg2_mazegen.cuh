@@ -24,7 +24,7 @@ struct MazeGrid {
     }
 };
 
-PG2_DEV_NOINLINE MazeGrid kruskal_maze(WarpCtx& w, int mw, int mh) {
+PG2_TU_LOCAL PG2_DEV_NOINLINE MazeGrid kruskal_maze(WarpCtx& w, int mw, int mh) {
     const int lane = w.lane;
     MazeGrid m;
     m.mw = mw; m.mh = mh; m.aw = mw + 2; m.ah = mh + 2;

@@ -6,6 +6,13 @@
 #pragma once
 #include <stdint.h>
 
+// engine_final.cu is linked beside engine.cu into one library and includes the same headers: the few non-template,
+// non-inline functions they define are static there (it defines PG2_TU_LOCAL as static), so that both translation units
+// do not define them. Empty everywhere else.
+#ifndef PG2_TU_LOCAL
+#define PG2_TU_LOCAL
+#endif
+
 #ifndef PG2_HOSTSIM
 #include <cuda_runtime.h>
 #define PG2_DEV __device__ __forceinline__

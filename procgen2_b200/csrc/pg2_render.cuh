@@ -166,7 +166,7 @@ struct FrameT {
 
 // Deterministic sin/cos in degrees, mirrored operation by operation from oracle/raster.c
 // (pg2o_sincos_deg): IEEE double add/mul only, fixed order, no FMA.
-PG2_DEV_CALL void sincos_deg(double deg, double* s, double* c) {
+PG2_TU_LOCAL PG2_DEV_CALL void sincos_deg(double deg, double* s, double* c) {
     double r = fmod(deg, 360.0);
     if (r < 0.0) r = __dadd_rn(r, 360.0);
     int q = (int)__ddiv_rn(__dadd_rn(r, 45.0), 90.0);

@@ -165,7 +165,7 @@ struct WarpMt {
 };
 
 // rng.seed(seed): mt[0] = seed; mt[i] = 1812433253 * (mt[i-1] ^ (mt[i-1] >> 30)) + i; position = 624.
-PG2_DEV_NOINLINE void mt_seed(uint32_t* mt, uint32_t seed) {
+PG2_TU_LOCAL PG2_DEV_NOINLINE void mt_seed(uint32_t* mt, uint32_t seed) {
     uint32_t x = seed;
     mt[0] = x;
     for (int i = 1; i < MT_N; i++) {

@@ -21,10 +21,17 @@ GAMES = ("bossfight", "caveflyer", "chaser", "climber", "coinrun", "jumper", "ma
 class _Config(ctypes.Structure):
     _fields_ = [("game", ctypes.c_char_p), ("num_envs", ctypes.c_int32), ("seed", ctypes.c_int32),
                 ("first_env", ctypes.c_int32), ("device", ctypes.c_int32), ("max_episode_steps", ctypes.c_int32),
-                ("assets_path", ctypes.c_char_p), ("auto_reset", ctypes.c_int32), ("distribution_mode", ctypes.c_int32)]
+                ("assets_path", ctypes.c_char_p), ("auto_reset", ctypes.c_int32), ("distribution_mode", ctypes.c_int32),
+                ("final_obs", ctypes.c_int32)]
 
 
 _lib = None
+
+
+class _Raw:
+    """A device buffer of the engine, described for torch.as_tensor (__cuda_array_interface__)."""
+    def __init__(self, ptr, shape, typestr):
+        self.__cuda_array_interface__ = {"shape": shape, "typestr": typestr, "data": (ptr, False), "version": 2}
 
 
 def load_library():
@@ -48,7 +55,8 @@ def load_library():
     L.pg2_fetch.argtypes = [vp, vp, vp, vp, vp]
     L.pg2_step_pipelined.argtypes = [vp, vp, vp, vp, vp, vp]
     L.pg2_pipeline_flush.argtypes = [vp]
-    for name in ("pg2_obs_device", "pg2_reward_device", "pg2_terminated_device", "pg2_truncated_device", "pg2_stream"):
+    L.pg2_fetch_final.argtypes = [vp, vp]
+    for name in ("pg2_obs_device", "pg2_reward_device", "pg2_terminated_device", "pg2_truncated_device", "pg2_final_obs_device", "pg2_stream"):
         getattr(L, name).argtypes = [vp]
         getattr(L, name).restype = vp
     L.pg2_sync.argtypes = [vp]
@@ -82,20 +90,25 @@ class BatchedEnv:
     """N environments of one game on one GPU.
 
     env i is seeded ``seed + first_env + i`` and reproduces a reference process created with
-    that seed (cenv_make -> cenv_reset -> cenv_step..., reset on terminate)."""
+    that seed (cenv_make -> cenv_reset -> cenv_step..., reset on terminate).
+
+    final_obs=True (needs auto_reset): the engine also keeps the terminal frame of every env that finishes, the frame the
+    reference returns from cenv_step before its caller resets it; read it with final_obs_view() or fetch_final()."""
 
     def __init__(self, game, num_envs, seed=0, device=0, first_env=0, max_episode_steps=0, assets_path=None, auto_reset=True,
-                 distribution_mode=-1):
+                 distribution_mode=-1, final_obs=False):
         L = load_library()
         self.game, self.num_envs, self.device = game, int(num_envs), int(device)
         self._assets = assets_path.encode() if assets_path else None
         cfg = _Config(game.encode(), self.num_envs, int(np.int32(np.uint32(seed & 0xffffffff))), int(first_env), self.device,
-                      int(max_episode_steps), self._assets, 1 if auto_reset else 0, int(distribution_mode))
+                      int(max_episode_steps), self._assets, 1 if auto_reset else 0, int(distribution_mode), 1 if final_obs else 0)
         h = ctypes.c_void_p()
         _check(L.pg2_create(ctypes.byref(cfg), ctypes.byref(h)))
         self._h = h
         self._L = L
+        self.final_obs = bool(final_obs)
         self._torch_views = None
+        self._final_view = None
 
     # ---- host-buffer API (numpy) -------------------------------------------------------------
     def reset(self, seeds=None):
@@ -125,6 +138,13 @@ class BatchedEnv:
         _check(self._L.pg2_fetch(self._h, *(x.ctypes.data if x is not None else None for x in (o, r, t, tr))))
         return o, r, (t.astype(bool) if t is not None else None), (tr.astype(bool) if tr is not None else None)
 
+    def fetch_final(self):
+        """Blocking copy of the terminal-frame buffer (final_obs engines): uint8 [N, 64, 64, 3]. Row e is the terminal frame
+        of env e's last finished episode, written in the step it finished in (zero before any)."""
+        out = np.empty((self.num_envs,) + OBS_SHAPE, np.uint8)
+        _check(self._L.pg2_fetch_final(self._h, out.ctypes.data))
+        return out
+
     def fetch_into(self, obs=None, reward=None, terminated=None, truncated=None):
         _check(self._L.pg2_fetch(self._h, *(x.ctypes.data if x is not None else None for x in (obs, reward, terminated, truncated))))
 
@@ -148,17 +168,23 @@ class BatchedEnv:
         aliasing the engine's HBM buffers (zero copy, via __cuda_array_interface__)."""
         if self._torch_views is None:
             import torch
-
-            class _Raw:
-                def __init__(self, ptr, shape, typestr):
-                    self.__cuda_array_interface__ = {"shape": shape, "typestr": typestr, "data": (ptr, False), "version": 2}
-
             n = self.num_envs
             dev = torch.device("cuda", self.device)
             mk = lambda fn, shape, ts: torch.as_tensor(_Raw(fn(self._h), shape, ts), device=dev)
             self._torch_views = (mk(self._L.pg2_obs_device, (n,) + OBS_SHAPE, "|u1"), mk(self._L.pg2_reward_device, (n,), "<f4"),
                                  mk(self._L.pg2_terminated_device, (n,), "|u1"), mk(self._L.pg2_truncated_device, (n,), "|u1"))
         return self._torch_views
+
+    def final_obs_view(self):
+        """The terminal-frame buffer of a final_obs engine (uint8 [N, 64, 64, 3], what fetch_final copies) as a CUDA tensor
+        aliasing the engine's HBM buffer, like torch_views(); None without final_obs."""
+        if not self.final_obs:
+            return None
+        if self._final_view is None:
+            import torch
+            raw = _Raw(self._L.pg2_final_obs_device(self._h), (self.num_envs,) + OBS_SHAPE, "|u1")
+            self._final_view = torch.as_tensor(raw, device=torch.device("cuda", self.device))
+        return self._final_view
 
     def step_torch(self, actions):
         """actions: int32 CUDA tensor (num_envs,) on this engine's device."""

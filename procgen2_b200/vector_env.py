@@ -8,7 +8,9 @@ Conventions (Gymnasium 1.x vector API):
   * `reset(seed=None, options=None) -> (obs, info)`, `step(actions) -> (obs, reward, terminated, truncated, info)`;
   * autoreset mode SAME_STEP: an env that terminates or is truncated is reset on device inside the same step, the
     returned observation is the first frame of the new episode (the reference's caller does the same by hand:
-    "if terminated: obs = reset()", game_test.py:38-40);
+    "if terminated: obs = reset()", game_test.py:38-40). With `final_obs=True` the step's info also holds the frame the
+    episode ended in, as Gymnasium 1.x's same-step autoreset does: `info["final_obs"]` (uint8 [num_envs, 64, 64, 3]; row
+    e is valid where `info["_final_obs"][e]`, i.e. where env e terminated or was truncated in this step);
   * `seed`: int -> env i restarts its RNG stream from seed + i (cenv_reset option "seed", coinrun.cpp:313-317), or a
     sequence of num_envs ints; None continues the streams;
   * the returned tensors are views of buffers the next step overwrites: `.clone()` what must outlive a step
@@ -63,16 +65,18 @@ class ProcgenVectorEnv(_VectorEnvBase):
 
     DISTRIBUTION_MODES = {None: -1, "default": -1, "easy": 0, "hard": 1, "memory": 2, "extreme": 2}
 
-    def __init__(self, game, num_envs, seed=0, device=0, max_episode_steps=0, first_env=0, copy=False, distribution_mode=None):
+    def __init__(self, game, num_envs, seed=0, device=0, max_episode_steps=0, first_env=0, copy=False, distribution_mode=None,
+                 final_obs=False):
         """distribution_mode: None (the mode the reference compiles in), "easy" / "hard" / "memory" / "extreme" or the integer
-        of the reference's `Distribution_Mode` enum (games/<g>/tilemap.h); a mode the game does not have raises."""
+        of the reference's `Distribution_Mode` enum (games/<g>/tilemap.h); a mode the game does not have raises.
+        final_obs: return the terminal observations of finished envs in the step's info (see the module docstring)."""
         import torch
         self._torch = torch
         mode = self.DISTRIBUTION_MODES.get(distribution_mode, distribution_mode) if not isinstance(distribution_mode, int) else distribution_mode
         if not isinstance(mode, int):
             raise ValueError("distribution_mode %r: expected one of %s or an integer" % (distribution_mode, sorted(k for k in self.DISTRIBUTION_MODES if k)))
         self.env = BatchedEnv(game, num_envs, seed=seed, device=device, first_env=first_env, max_episode_steps=max_episode_steps,
-                              distribution_mode=mode)
+                              distribution_mode=mode, final_obs=final_obs)
         self.game, self.num_envs, self.copy = game, int(num_envs), bool(copy)
         self.device = torch.device("cuda", device)
         self.stream = torch.cuda.ExternalStream(self.env.stream_ptr, device=self.device)
@@ -87,6 +91,7 @@ class ProcgenVectorEnv(_VectorEnvBase):
             self.observation_space = _Box(0, 255, (self.num_envs,) + OBS_SHAPE, np.uint8)
             self.action_space = _MultiDiscrete([NUM_ACTIONS] * self.num_envs)
         self._obs, self._reward, self._terminated, self._truncated = self.env.torch_views()
+        self._final_obs = self.env.final_obs_view()
         self._actions = torch.empty(self.num_envs, dtype=torch.int32, device=self.device)
         self._done_event = torch.cuda.Event()
 
@@ -123,7 +128,10 @@ class ProcgenVectorEnv(_VectorEnvBase):
             self._actions.copy_(actions.view(-1), non_blocking=True)
             self.env.step_torch(self._actions)
         obs, reward, terminated, truncated = self._publish()
-        return obs, reward, terminated, truncated, {}
+        info = {}
+        if self._final_obs is not None:
+            info = {"final_obs": self._final_obs.clone() if self.copy else self._final_obs, "_final_obs": terminated | truncated}
+        return obs, reward, terminated, truncated, info
 
     # ---- interchange -----------------------------------------------------------------------------------------------
     def dlpack(self):
