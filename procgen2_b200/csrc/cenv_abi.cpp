@@ -89,19 +89,22 @@ void publish_device_pointers() {
     }
 }
 
-// results of the last step / reset -> host buffers. Every device's copies are enqueued first (asynchronous, pinned
-// destination), then waited for: the transfers of different devices overlap.
-int fetch() {
-    for (size_t d = 0; d < g_engines.size(); d++) {
-        const size_t o = (size_t)g_first[d];
-        if (pg2_fetch_async(g_engines[d], g_host_copy ? g_obs + o * kObsBytes : nullptr, g_reward + o, g_term + o, g_trunc + o)) {
-            fprintf(stderr, "[procgen2_b200] %s\n", pg2_last_error());
-            return 1;
-        }
-    }
+// copy(engine, its first env) is enqueued on every device first (asynchronous, pinned destination), then every device is
+// waited for: the transfers of different devices overlap.
+template <class F>
+int enqueue_then_sync(F copy) {
+    for (size_t d = 0; d < g_engines.size(); d++)
+        if (copy(g_engines[d], (size_t)g_first[d])) { fprintf(stderr, "[procgen2_b200] %s\n", pg2_last_error()); return 1; }
     for (size_t d = 0; d < g_engines.size(); d++)
         if (pg2_sync(g_engines[d])) { fprintf(stderr, "[procgen2_b200] %s\n", pg2_last_error()); return 1; }
     return 0;
+}
+
+// results of the last step / reset -> host buffers
+int fetch() {
+    return enqueue_then_sync([](pg2_engine* e, size_t o) {
+        return pg2_fetch_async(e, g_host_copy ? g_obs + o * kObsBytes : nullptr, g_reward + o, g_term + o, g_trunc + o);
+    });
 }
 
 // "final_observation" with host_copy, after fetch(): the terminal frames of the envs that finished in the step -> the host
@@ -109,16 +112,7 @@ int fetch() {
 // older contents, as on the device.
 int fetch_final() {
     for (int e = 0; e < g_num_envs; e++) g_done[e] = g_term[e] | g_trunc[e];
-    for (size_t d = 0; d < g_engines.size(); d++) {
-        const size_t o = (size_t)g_first[d];
-        if (pg2_fetch_final_async(g_engines[d], g_done.data() + o, g_final_obs + o * kObsBytes)) {
-            fprintf(stderr, "[procgen2_b200] %s\n", pg2_last_error());
-            return 1;
-        }
-    }
-    for (size_t d = 0; d < g_engines.size(); d++)
-        if (pg2_sync(g_engines[d])) { fprintf(stderr, "[procgen2_b200] %s\n", pg2_last_error()); return 1; }
-    return 0;
+    return enqueue_then_sync([](pg2_engine* e, size_t o) { return pg2_fetch_final_async(e, g_done.data() + o, g_final_obs + o * kObsBytes); });
 }
 
 void destroy_all() {

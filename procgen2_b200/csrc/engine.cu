@@ -7,7 +7,7 @@
 //   k_reset<G>   warp-per-finished-env: reset() with on-device procedural level generation,
 //                continuing the env's MT19937 stream                <- reset()     (<g>.cpp)
 //   k_render<G>  CTA-per-env: 64x64x3 observation, TMA bulk store    <- render_game (<g>.cpp) + SDL
-// (final_obs engines draw the terminal frames of finished envs too: k_render_final<G>, engine_final.cu, see enqueue_step)
+// (final_obs engines draw the terminal frames of finished envs too: k_render<G, true>, engine_final.cu, see enqueue_step)
 // No CPU fallback exists: every entry point fails loudly when CUDA is unavailable.
 #include <cuda_runtime.h>
 #include <stdio.h>
@@ -153,14 +153,11 @@ __global__ void __launch_bounds__(32 * RESET_WARPS_PER_CTA) k_reset(typename G::
     }
 }
 
-// k_render_final<G> (engine_final.cu)
+// engine_final.cu. This unit never names k_render<G, true>: instantiating it here, even by taking its address, changes
+// the code of every k_render<G, false>.
 cudaError_t final_set_sort_table(const uint8_t* table);
 template <class G>
-cudaError_t render_final_occupancy(int* ctas_per_sm);
-template <class G>
-void launch_render_final(int grid, cudaStream_t on, const typename G::State& s, const CommonState& c, const TexInfo* tex, const uint32_t* atlas,
-                         uint8_t* obs, int* ticket, int mode, const int* list, const int* list_count, const uint8_t* pending, int N,
-                         uint8_t* view_cache, const SwapArgs& swap, uint8_t* final_obs, int* zero_ticket);
+const void* render_final_kernel();   // k_render<G, true>
 
 // ------------------------------------------------------------------------------------------------
 // host engine
@@ -206,7 +203,7 @@ struct EngineBase {
     int num_sms = 148;
     int step_epw = 1;          // environments per warp in k_step
     int render_ctas_per_sm = 8;   // resident CTAs of k_render per SM (occupancy query)
-    int final_ctas_per_sm = 8;    // ... of k_render_final (final_on)
+    int final_ctas_per_sm = 8;    // ... of k_render<G, true> (final_on)
     // device buffers
     void* state_mem = nullptr;
     void* common_mem = nullptr;
@@ -423,11 +420,11 @@ struct Engine : EngineBase {
         PG2_CUDA(cudaStreamSynchronize(stream));
         PG2_CUDA(cudaFuncSetAttribute(k_reset<G>, cudaFuncAttributeMaxDynamicSharedMemorySize, reset_smem()));
         // persistent render grid = exactly the CTAs that are resident at once (registers / shared memory decide)
-        PG2_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&render_ctas_per_sm, k_render<G>, RENDER_THREADS, 0));
+        PG2_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&render_ctas_per_sm, k_render<G, false>, RENDER_THREADS, 0));
         if (render_ctas_per_sm < 1) render_ctas_per_sm = 1;
         if (const char* o = getenv("PG2_RENDER_CTAS_PER_SM")) render_ctas_per_sm = atoi(o) > 0 ? atoi(o) : render_ctas_per_sm;
         if (final_on) {
-            PG2_CUDA(render_final_occupancy<G>(&final_ctas_per_sm));
+            PG2_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&final_ctas_per_sm, render_final_kernel<G>(), RENDER_THREADS, 0));
             if (final_ctas_per_sm < 1) final_ctas_per_sm = 1;
             if (const char* o = getenv("PG2_RENDER_CTAS_PER_SM")) final_ctas_per_sm = atoi(o) > 0 ? atoi(o) : final_ctas_per_sm;
         }
@@ -512,21 +509,22 @@ struct Engine : EngineBase {
     }
     // final: a step of a final_on engine. With level prefetch the render of the step draws the terminal frames too (mode 0);
     // without it, final is the pass over the reset list before k_reset (mode 2) that writes the terminal frames.
-    void launch_render(int mode, int* ticket, cudaStream_t on, bool final = false) {
+    int launch_render(int mode, int* ticket, cudaStream_t on, bool final = false) {
         const int per_sm = final ? final_ctas_per_sm : render_ctas_per_sm;
         int grid = N < num_sms * per_sm ? N : num_sms * per_sm;
         // (level prefetch: the list / counter k_step appended this step's finished envs to)
         const int* lst = prefetch && ka_list ? ka_list : reset_list;
         const int* cnt = prefetch && ka_count ? ka_count : reset_count + parity;
-        if (!final)
-            k_render<G><<<grid, RENDER_THREADS, 0, on>>>(st, common, texinfo, atlas, out[cur].obs, ticket, mode, lst, cnt, pending, N, view_cache, swap_args);
-        else if (prefetch)
-            launch_render_final<G>(grid, on, st, common, texinfo, atlas, out[cur].obs, ticket, mode, lst, cnt, pending, N, view_cache, swap_args,
-                                   out[cur].final_obs, nullptr);
-        else
-            launch_render_final<G>(grid, on, st, common, texinfo, atlas, out[cur].final_obs, ticket, mode, lst, cnt, pending, N, view_cache, swap_args,
-                                   nullptr, final_ticket + (parity ^ 1));
+        // final with prefetch: reset frames to obs, terminal frames to final_obs; final without: the terminal frames are obs
+        uint8_t* obs = final && !prefetch ? out[cur].final_obs : out[cur].obs;
+        uint8_t* final_obs = final && prefetch ? out[cur].final_obs : nullptr;
+        int* zero_ticket = final && !prefetch ? final_ticket + (parity ^ 1) : nullptr;
+        void* args[] = { &st, &common, &texinfo, &atlas, &obs, &ticket, &mode, &lst, &cnt, &pending, &N, &view_cache, &swap_args,
+                         &final_obs, &zero_ticket };
+        const void* kernel = final ? render_final_kernel<G>() : (const void*)k_render<G, false>;
+        PG2_CUDA(cudaLaunchKernel(kernel, dim3(grid), dim3(RENDER_THREADS), args, 0, on));
         launches++;
+        return 0;
     }
 
     int reset(const int32_t* seeds) override {
@@ -543,7 +541,7 @@ struct Engine : EngineBase {
         PG2_CUDA(cudaMemsetAsync(reset_count + 2, 0, 2 * sizeof(int), stream));
         PG2_CUDA(cudaMemsetAsync(pending, 0, N, stream));   // no env of the last step is waiting for its level swap any more
         ka_list = nullptr; ka_count = nullptr;              // ... and the render below has no swap list (reset_count[0..1] stay zero for these games)
-        launch_render(0, reset_count + 2, stream);
+        if (launch_render(0, reset_count + 2, stream)) return 1;
         PG2_CUDA(cudaMemsetAsync(out[cur].reward, 0, sizeof(float) * N, stream));
         PG2_CUDA(cudaMemsetAsync(out[cur].terminated, 0, N, stream));
         PG2_CUDA(cudaMemsetAsync(out[cur].truncated, 0, N, stream));
@@ -565,8 +563,8 @@ struct Engine : EngineBase {
     // render on the second stream; the wait for it and the tail render are not counted).
     // final_on: the terminal frame of a finished env is drawn from the state it finished in, before any reset touches it.
     // With level prefetch that state is still live when the render starts, and the render CTA that swaps the env's level
-    // in draws the terminal frame first (k_render_final, no extra launch). Otherwise k_reset overwrites it, so a pass of
-    // k_render_final over the reset list runs between k_step and k_reset (one more launch; its time counts as [1]). On the
+    // in draws the terminal frame first (k_render<G, true>, no extra launch). Otherwise k_reset overwrites it, so a pass of
+    // k_render<G, true> over the reset list runs between k_step and k_reset (one more launch; its time counts as [1]). On the
     // overlap_reset schedule the pass runs before the fork: after it, between the fork and k_reset, it would delay k_reset
     // until the render of the other envs, which fills the SMs meanwhile, has finished (chaser 4096: +55 % per step).
     // The pass's ticket alternates with the step parity: each pass zeroes the one the next step uses.
@@ -604,7 +602,7 @@ struct Engine : EngineBase {
         if (prof) prof_mark();
         if (launch_step(stream)) return 1;
         if (prof) prof_mark();
-        if (final_on && !prefetch) launch_render(2, final_ticket + parity, stream, true);
+        if (final_on && !prefetch && launch_render(2, final_ticket + parity, stream, true)) return 1;
         if (overlap_reset) {   // fork: the render of all OTHER envs runs on the second stream
             PG2_CUDA(cudaEventRecord(ev_stepped, stream));
             PG2_CUDA(cudaStreamWaitEvent(reset_stream, ev_stepped, 0));
@@ -615,13 +613,13 @@ struct Engine : EngineBase {
         if (prof) prof_mark();
         if (overlap_reset) {
             if (prof) prof_mark_on(reset_stream);
-            launch_render(1, reset_count + 2, reset_stream);
+            if (launch_render(1, reset_count + 2, reset_stream)) return 1;
             if (prof) prof_mark_on(reset_stream);
             PG2_CUDA(cudaEventRecord(ev_reset_done, reset_stream));   // = main render done
             PG2_CUDA(cudaStreamWaitEvent(stream, ev_reset_done, 0));
-            launch_render(2, reset_count + 3, stream);
+            if (launch_render(2, reset_count + 3, stream)) return 1;
         } else {
-            launch_render(0, reset_count + 2, stream, final_on && prefetch);
+            if (launch_render(0, reset_count + 2, stream, final_on && prefetch)) return 1;
         }
         if (prof) prof_mark();
         return 0;

@@ -34,7 +34,10 @@ struct SimBase {
     struct FieldInfo { std::string name; void* ptr; int esz, per_env; bool env_major; };
     std::vector<FieldInfo> fields;
     int N = 0, max_episode_steps = 0;
-    std::vector<uint8_t> obs, terminated, truncated;
+    // the engine's step variants: auto_reset = false (pg2_config::auto_reset = 0) does not reset a finished env; final_on
+    // (pg2_config::final_obs) draws the terminal frame of a finished env into final_obs before the reset
+    bool auto_reset = true, final_on = false;
+    std::vector<uint8_t> obs, terminated, truncated, final_obs;
     std::vector<float> reward;
 };
 
@@ -95,7 +98,8 @@ struct Sim : SimBase {
     void step(const int32_t* actions) override {
         for (int e = 0; e < N; e++) {
             bool done = step_body<G>(st, c, e, actions[e], reward.data(), terminated.data(), truncated.data(), max_episode_steps, StepCtx{ 0, 1 });
-            if (done) reset_body<G>(st, c, e, mt_scratch.data(), arena.data(), 0);
+            if (done && final_on) render_body<G>(st, c, e, *frame, tex, atlas, final_obs.data(), G::STATIC_VIEW ? view_cache.data() : nullptr);
+            if (done && auto_reset) reset_body<G>(st, c, e, mt_scratch.data(), arena.data(), 0);
             render(e);
         }
     }
@@ -117,9 +121,10 @@ extern "C" {
 const char* hs_last_error() { return g_err.c_str(); }
 void hs_debug_counters(long* out) { out[0] = pg2::g_dbg_slow; out[1] = pg2::g_dbg_quads; out[2] = pg2::g_dbg_quads_slow; out[3] = pg2::g_dbg_rb; }
 
-void* hs_create_mode(const char* game, int n, int seed, int max_ep, const char* assets, int mode);
-void* hs_create(const char* game, int n, int seed, int max_ep, const char* assets) { return hs_create_mode(game, n, seed, max_ep, assets, -1); }
-void* hs_create_mode(const char* game, int n, int seed, int max_ep, const char* assets, int mode) {
+// mode: the distribution mode (-1: the game's default). auto_reset / final_obs: the step variants (SimBase); final_obs
+// needs auto_reset (like pg2_create): NULL otherwise.
+void* hs_create(const char* game, int n, int seed, int max_ep, const char* assets, int mode, int auto_reset, int final_obs) {
+    if (final_obs && !auto_reset) { g_err = "final_obs needs auto_reset = 1"; return nullptr; }
     std::string g = game;
     if (g_sort_table.empty()) { g_sort_table = build_sort_perm(SORT_MAXN); g_sort_perm = g_sort_table.data(); }
     SimBase* out = nullptr;
@@ -134,6 +139,9 @@ void* hs_create_mode(const char* game, int n, int seed, int max_ep, const char* 
 #undef PG2_TRY_GAME
     if (!out) { g_err = "unknown game " + g; return nullptr; }
     if (!ok) { delete out; return nullptr; }
+    out->auto_reset = auto_reset != 0;
+    out->final_on = final_obs != 0;
+    if (out->final_on) out->final_obs.assign((size_t)n * OBS_BYTES, 0);
     return out;
 }
 void hs_destroy(void* h) { delete (SimBase*)h; }
@@ -145,6 +153,9 @@ const uint8_t* hs_obs(void* h) { return ((SimBase*)h)->obs.data(); }
 const float* hs_reward(void* h) { return ((SimBase*)h)->reward.data(); }
 const uint8_t* hs_terminated(void* h) { return ((SimBase*)h)->terminated.data(); }
 const uint8_t* hs_truncated(void* h) { return ((SimBase*)h)->truncated.data(); }
+// The terminal frames of a sim created with final_obs: N * 12288 bytes, row e written in the steps env e finished in.
+// NULL for a sim without final_obs.
+const uint8_t* hs_final_obs(void* h) { SimBase* s = (SimBase*)h; return s->final_on ? s->final_obs.data() : nullptr; }
 long hs_read_field(void* h, const char* name, void* out, long capacity, int* elem_size, int* per_env) {
     SimBase* s = (SimBase*)h;
     void* ptr; int esz, pe;

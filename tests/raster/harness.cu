@@ -64,7 +64,7 @@ static int run_frames(int npass, int nenv, const sc_scene* scenes, const TexInfo
     RH_CUDA(cudaMemcpy(atlas, atlas_h, sizeof(uint32_t) * natlas, cudaMemcpyHostToDevice));
     if (grid <= 0) {
         int per_sm = 0, dev = 0, sms = 0;
-        RH_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_render<S>, RENDER_THREADS, 0));
+        RH_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_render<S, false>, RENDER_THREADS, 0));
         RH_CUDA(cudaGetDevice(&dev));
         RH_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
         grid = nenv < sms * per_sm ? nenv : sms * per_sm;
@@ -81,7 +81,7 @@ static int run_frames(int npass, int nenv, const sc_scene* scenes, const TexInfo
         RH_CUDA(cudaMemcpy(c.view_valid, valid.data(), nenv, cudaMemcpyHostToDevice));
         RH_CUDA(cudaMemset(c.fault, 0, sizeof(int32_t) * nenv));
         RH_CUDA(cudaMemset(ticket, 0, sizeof(int)));
-        k_render<S><<<grid, RENDER_THREADS>>>(s, c, tex, atlas, obs, ticket, 0, nullptr, nullptr, nullptr, nenv, cache, swap);
+        k_render<S, false><<<grid, RENDER_THREADS>>>(s, c, tex, atlas, obs, ticket, 0, nullptr, nullptr, nullptr, nenv, cache, swap, nullptr, nullptr);
         RH_CUDA(cudaGetLastError());
         RH_CUDA(cudaDeviceSynchronize());
         RH_CUDA(cudaMemcpy(obs_out + (size_t)p * nenv * OBS_BYTES, obs, (size_t)nenv * OBS_BYTES, cudaMemcpyDeviceToHost));

@@ -18,14 +18,13 @@ def lib():
         from tests.hostsim import build as hb
         L = ctypes.CDLL(hb.build())
         L.hs_create.restype = ctypes.c_void_p
-        L.hs_create.argtypes = [ctypes.c_char_p, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_char_p]
-        L.hs_create_mode.restype = ctypes.c_void_p
-        L.hs_create_mode.argtypes = [ctypes.c_char_p, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_char_p, ctypes.c_int]
+        L.hs_create.argtypes = [ctypes.c_char_p, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_char_p] + [ctypes.c_int] * 3
         L.hs_destroy.argtypes = [ctypes.c_void_p]
         L.hs_reset.argtypes = [ctypes.c_void_p, ctypes.c_void_p]
         L.hs_step.argtypes = [ctypes.c_void_p, ctypes.c_void_p]
         L.hs_render_human.argtypes = [ctypes.c_void_p, ctypes.c_int, ctypes.c_int, ctypes.c_int, ctypes.c_void_p]
-        for n, t in (("hs_obs", ctypes.c_uint8), ("hs_reward", ctypes.c_float), ("hs_terminated", ctypes.c_uint8), ("hs_truncated", ctypes.c_uint8)):
+        for n, t in (("hs_obs", ctypes.c_uint8), ("hs_reward", ctypes.c_float), ("hs_terminated", ctypes.c_uint8), ("hs_truncated", ctypes.c_uint8),
+                     ("hs_final_obs", ctypes.c_uint8)):
             getattr(L, n).restype = ctypes.POINTER(t)
             getattr(L, n).argtypes = [ctypes.c_void_p]
         L.hs_read_field.restype = ctypes.c_long
@@ -41,10 +40,14 @@ def lib():
 
 
 class HostSim:
-    def __init__(self, game, num_envs, seed, max_episode_steps=0, distribution_mode=-1):
+    """auto_reset / final_obs: the engine's step variants (pg2_config). auto_reset=False: a finished env is not reset;
+    final_obs=True: final_obs() = the terminal frame of every env that finished, written in the step it finished in."""
+
+    def __init__(self, game, num_envs, seed, max_episode_steps=0, distribution_mode=-1, auto_reset=True, final_obs=False):
         L = lib()
         self.n = num_envs
-        self.h = L.hs_create_mode(game.encode(), num_envs, seed, max_episode_steps, ASSETS.encode(), distribution_mode)
+        self.h = L.hs_create(game.encode(), num_envs, seed, max_episode_steps, ASSETS.encode(), distribution_mode,
+                             1 if auto_reset else 0, 1 if final_obs else 0)
         if not self.h:
             raise RuntimeError(L.hs_last_error().decode())
 
@@ -57,6 +60,9 @@ class HostSim:
 
     def truncated(self):
         return np.ctypeslib.as_array(lib().hs_truncated(self.h), shape=(self.n,)).copy().astype(bool)
+
+    def final_obs(self):
+        return np.ctypeslib.as_array(lib().hs_final_obs(self.h), shape=(self.n, 64, 64, 3)).copy()
 
     def reset(self, seeds=None):
         if seeds is not None:
